@@ -3,12 +3,16 @@
 reference's CPU path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one complete sort of the workload (histogram + setup + every live scatter pass)
 through the C ABI (librsx.so).  The input is restored from a pristine device copy OUTSIDE the
 timed region before every step (the reference's own Google-Benchmark loop forgets to do this,
 radix_bench.cpp:91-93, SURVEY.md §6); each step is timed with CUDA events on the launch stream.
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+
+--dump-outputs DIR writes a fixed, seeded sample of what the last timed step returned, per
+workload, so that two builds can be compared output for output (see dump_sample).
 """
 from __future__ import annotations
 
@@ -230,6 +234,30 @@ def load_traffic(kb):
     return None, None
 
 
+DUMP_SEED = 20261020
+DUMP_SAMPLE = 1 << 20  # positions per workload: two workloads of <= 8-byte keys stay under 48 MiB
+
+
+def dump_sample(out_dir, workload, res):
+    """Writes DIR/<workload>_sorted.npy: the key bits of the sorted output at a fixed, seeded sample
+    of positions (all of them for small n).  Each 32-bit word is one float64 (exact), an 8-byte key
+    gives two columns, low word first: equal arrays mean equal bytes, NaN bit patterns of float
+    keys included.  DIR/<workload>_index.npy holds the sampled positions; it carries no output
+    and is the same in every build, it only says where each row of _sorted was read."""
+    import numpy as np
+    import torch
+    n = res.numel()
+    if n <= DUMP_SAMPLE:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, size=DUMP_SAMPLE, dtype=np.int64))
+    vals = res[torch.from_numpy(idx).to(res.device)].cpu().numpy()
+    words = vals.view(np.uint32).reshape(idx.shape[0], -1)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{workload}_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, f"{workload}_sorted.npy"), words.astype(np.float64))
+
+
 def bench_single(args, rsx, torch, workload, dev, steps, warmup, do_e2e, do_cpu):
     """One workload on one GPU: device-resident steps (value), per-kernel roofline, optional e2e
     through host buffers and the CPU reference beside it.  Returns the JSON-able dict."""
@@ -295,6 +323,8 @@ def bench_single(args, rsx, torch, workload, dev, steps, warmup, do_e2e, do_cpu)
     d1, s1, x1 = rsx.verify(res, kf)
     verified = d1 == 0 and (s1, x1) == (s0, x0)
     assert verified, "timed result is not a sorted permutation of the input"
+    if args.dump_outputs:
+        dump_sample(args.dump_outputs, workload, res)
 
     ms_per_step = sum(times) / len(times)
     value = n / (ms_per_step * 1e-3) / 1e9
@@ -338,7 +368,7 @@ def bench_single(args, rsx, torch, workload, dev, steps, warmup, do_e2e, do_cpu)
         h_src = torch.empty(n, dtype=tdt, pin_memory=True)
         h_aux = torch.empty(n, dtype=tdt, pin_memory=True)
         h_pristine = pristine.cpu()
-        e2e_steps = max(5, steps)
+        e2e_steps = steps
         e2e_times = []
         for i in range(1 + e2e_steps):
             h_src.copy_(h_pristine)
@@ -481,7 +511,14 @@ def main():
     ap.add_argument("--no-fused", action="store_true", help="N > 1: NCCL all_to_all instead of fused peer stores")
     ap.add_argument("--rank-mode", type=int, default=-1, help="-1 auto (hardware probe), 0 ticket, 1 ballot")
     ap.add_argument("--variant", type=int, default=0, help="scatter tuning variant (rsx_scatter.cuh)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of each workload's last timed output to DIR/*.npy "
+                         "(one-GPU runs only; refused under torchrun, --impl reference and --sweep)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.sweep or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs applies to the one-GPU timed sort only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -524,7 +561,7 @@ def main():
         if not explicit_workload and not args.no_extra:
             for key, wl in (("config5_u64", "2B-u64-uniform"), ("config5_u64_zipf", "2B-u64-zipf")):
                 a2 = copy.copy(args)
-                a2.workload, a2.steps, a2.warmup, a2.no_e2e = wl, min(args.steps, 3), 3, True
+                a2.workload, a2.warmup, a2.no_e2e = wl, 3, True
                 t2, n2, d2, m2, o2, _ = WORKLOADS[wl]
                 torch.cuda.empty_cache()
                 r2 = dsort.bench_partitioned(a2, rsx, t2, n2, d2, m2, o2, rank, world, dev,
@@ -544,8 +581,8 @@ def main():
 
     out = bench_single(args, rsx, torch, args.workload, dev, args.steps, args.warmup, not args.no_e2e, not args.no_cpu)
     if not explicit_workload and not args.no_extra:
-        # the u64 half of BASELINE's "u32/u64" metric, same contract, fewer steps
-        r64 = bench_single(args, rsx, torch, "1B-u64-uniform", dev, min(args.steps, 5), 3, False, False)
+        # the u64 half of BASELINE's "u32/u64" metric, same contract
+        r64 = bench_single(args, rsx, torch, "1B-u64-uniform", dev, args.steps, 3, False, False)
         out["u64_1B"] = {k: r64[k] for k in ("value", "unit", "ms_per_step", "steps", "dtype", "config", "roofline",
                                               "gpu_launches", "clocks")}
     print(json.dumps(out))
