@@ -92,6 +92,34 @@ int rsx_sort(void *src, void *aux, size_t n, const rsx_layout *layout, void **re
 int rsx_sort_rank(const void *src, void *index_buffer, size_t n, const rsx_layout *layout,
                   int idx_bytes, void **result, rsx_report *report, void *stream);
 
+/* ---- segmented sort: many independent arrays in one call ----------------------------------
+ * No reference equivalent (the reference sorts one array per call); what CUB's segmented sort and
+ * torch.sort(dim=-1) offer.  `offsets` holds nseg + 1 non-decreasing record offsets, offsets[0] == 0,
+ * offsets[nseg] == n; segment s is records [offsets[s], offsets[s+1]).  It may be a HOST or a
+ * DEVICE pointer (a device array is read back once); host offsets are checked before any device work.
+ *   content  every segment ends up exactly as radix_sort / radix_sort_rank of that segment alone
+ *            would leave it: stable by derived key, any KDF and RSX_FLAG_INVERT.  Rank indices are
+ *            relative to the segment's start (what torch.sort(dim=-1) returns).
+ *   result   ONE pointer for the batch, by the reference's parity rule applied to the batch: a column
+ *            is live if its digit is not the same in all n records; *result is src (index_buffer) if
+ *            the number of live columns is even, else aux (index_buffer + n).  A segment that is
+ *            trivial in a column live for the batch still goes through that pass, which for a stable
+ *            sort changes nothing.
+ *   early    only if every segment is already ordered (descents across a segment boundary do not
+ *            count): nothing moves and *result = src; a rank sort writes the segment-relative
+ *            identity into the first half and *result = index_buffer.
+ *   report   describes the batch (early_exit, ncols, live_mask, result_in_aux, kernel_launches).
+ * src / aux / index_buffer must be device (or managed) memory (RSX_ERR_MIXED_MEMORY otherwise), record
+ * sizes 1, 2, 4, 8 or 16 bytes (RSX_ERR_INVALID otherwise); idx_bytes must hold the longest segment's
+ * length - 1 (RSX_ERR_IDX_RANGE).  n < 2 returns src without touching the device, as rsx_sort does
+ * (a rank sort does what rsx_sort_rank does).  Synchronous like rsx_sort.  Short segments cost two
+ * kernel launches per batch however many there are; a segment longer than one CTA holds is sorted
+ * by the rsx_sort / rsx_sort_rank path on its own (DESIGN.md "Segmented sort"). */
+int rsx_sort_segments(void *src, void *aux, size_t n, const uint64_t *offsets, size_t nseg,
+                      const rsx_layout *layout, void **result, rsx_report *report, void *stream);
+int rsx_sort_rank_segments(const void *src, void *index_buffer, size_t n, const uint64_t *offsets, size_t nseg,
+                           const rsx_layout *layout, int idx_bytes, void **result, rsx_report *report, void *stream);
+
 /* ---- the two halves of the path, exposed for parity tests and profiling --------------------
  * rsx_histogram = phase 1-3 of rs_sort_main (radix_sort.hpp:46-80): one read of the keys
  * producing all key_bytes x 256 digit counts (column-major, BEFORE the exclusive scan, bins

@@ -8,6 +8,7 @@ torch tensors (torch is used for device memory and streams only):
 
     radix_sort(src, aux, n=None, kf=None)            -> radix_sort.hpp:98-115
     radix_sort_rank(src, index_buffer, n=None, kf=None) -> radix_sort_rank.hpp:97-112
+    radix_sort_segments / radix_sort_rank_segments        -> many independent arrays in one call
 
 Both return the tensor / half that holds the result, like the reference returns a pointer.
 There is NO CPU fallback: importing this module without a built ``librsx.so`` raises, and
@@ -35,7 +36,7 @@ RSX_ERR_WORKSPACE, RSX_ERR_IDX_RANGE, RSX_ERR_MIXED_MEMORY = -4, -5, -6
 
 #: every symbol include/rsx.h declares (tests check that the library exports all of them)
 EXPORTS = [
-    "rsx_sort", "rsx_sort_rank", "rsx_histogram", "rsx_histogram_column", "rsx_scatter_pass", "rsx_scatter_pass_to",
+    "rsx_sort", "rsx_sort_rank", "rsx_sort_segments", "rsx_sort_rank_segments", "rsx_histogram", "rsx_histogram_column", "rsx_scatter_pass", "rsx_scatter_pass_to",
     "rsx_split_counts", "rsx_split_pass_to", "rsx_scatter_pass_append", "rsx_histogram_column_sampled", "rsx_sample_keys", "rsx_plan_compaction",
     "rsx_multi_route", "rsx_multi_splitters", "rsx_sort_shard", "rsx_sort_multi",
     "rsx_workspace_bytes",
@@ -133,6 +134,10 @@ def _lib() -> C.CDLL:
     L.rsx_sort.argtypes = [vp, vp, sz, LP, C.POINTER(vp), RP, vp]
     L.rsx_sort_rank.restype = C.c_int
     L.rsx_sort_rank.argtypes = [vp, vp, sz, LP, C.c_int, C.POINTER(vp), RP, vp]
+    L.rsx_sort_segments.restype = C.c_int
+    L.rsx_sort_segments.argtypes = [vp, vp, sz, u64p, sz, LP, C.POINTER(vp), RP, vp]
+    L.rsx_sort_rank_segments.restype = C.c_int
+    L.rsx_sort_rank_segments.argtypes = [vp, vp, sz, u64p, sz, LP, C.c_int, C.POINTER(vp), RP, vp]
     L.rsx_histogram.restype = C.c_int
     L.rsx_histogram.argtypes = [vp, sz, LP, u64p, u64p, RP, vp]
     L.rsx_histogram_column.restype = C.c_int
@@ -310,6 +315,71 @@ def radix_sort_rank(src, index_buffer, n: Optional[int] = None, kf: Optional[Key
     flat = index_buffer.view(-1)
     off = (res.value - index_buffer.data_ptr()) // ib_bytes if n else 0
     return flat[off:off + n]
+
+
+def _offsets(offsets):
+    """offsets (int64 tensor on the CPU or a device, or a sequence of ints) -> (pointer, nseg, keep-alive)."""
+    torch = _torch()
+    if not isinstance(offsets, torch.Tensor):
+        offsets = torch.tensor([int(x) for x in offsets], dtype=torch.int64)
+    if offsets.dtype not in (torch.int64, torch.uint64) or offsets.dim() != 1 or offsets.numel() < 1:
+        raise ValueError("offsets must be a 1-D int64 tensor or a sequence of nseg + 1 ints")
+    offsets = offsets.contiguous()
+    return C.cast(C.c_void_p(offsets.data_ptr()), C.POINTER(C.c_uint64)), offsets.numel() - 1, offsets
+
+
+def radix_sort_segments(src, aux, offsets, kf: Optional[KeyFunc] = None, *, report: Optional[RsxReport] = None):
+    """Sorts every segment [offsets[s], offsets[s+1]) of `src` independently, in one call
+    (rsx_sort_segments).  `src`/`aux`: device tensors of the same dtype, n = offsets[-1] records
+    each; `offsets`: int64 tensor (CPU or CUDA) or a sequence of nseg + 1 ints.  Returns `src` or
+    `aux`, whichever holds the whole sorted batch (the reference's parity rule over the batch)."""
+    torch = _torch()
+    _check(src, "src"), _check(aux, "aux")
+    if src.dtype != aux.dtype or src.device != aux.device:
+        raise ValueError("src and aux must have the same dtype and device")
+    kf = kf or default_kdf(src.dtype)
+    L = kf.layout(src.element_size())
+    count = src.numel() * src.element_size() // L.record_bytes
+    off, nseg, keep = _offsets(offsets)
+    n = int(keep[-1])
+    if n > count or aux.numel() * aux.element_size() < n * L.record_bytes:
+        raise ValueError("offsets[-1] exceeds the buffers")
+    res = C.c_void_p()
+    rep = report if report is not None else RsxReport()
+    with torch.cuda.device(src.device if src.is_cuda else None):
+        st = _lib().rsx_sort_segments(src.data_ptr(), aux.data_ptr(), n, off, nseg, C.byref(L), C.byref(res),
+                                      C.byref(rep), _stream_ptr(src))
+    if st != RSX_OK:
+        raise RsxError(st, "rsx_sort_segments")
+    return aux if (n and res.value == aux.data_ptr() and res.value != src.data_ptr()) else src
+
+
+def radix_sort_rank_segments(src, index_buffer, offsets, kf: Optional[KeyFunc] = None, *,
+                             report: Optional[RsxReport] = None):
+    """Segment-relative stable argsort of every segment of `src` in one call (rsx_sort_rank_segments).
+    `index_buffer` has 2n entries; returns the n-entry half that holds the ranks.  `src` is not
+    modified."""
+    torch = _torch()
+    _check(src, "src"), _check(index_buffer, "index_buffer")
+    if src.device != index_buffer.device:
+        raise ValueError("src and index_buffer must be on the same device")
+    kf = kf or default_kdf(src.dtype)
+    L = kf.layout(src.element_size())
+    count = src.numel() * src.element_size() // L.record_bytes
+    off, nseg, keep = _offsets(offsets)
+    n = int(keep[-1])
+    if n > count or index_buffer.numel() < 2 * n:
+        raise ValueError("index_buffer must hold 2n entries")
+    ib_bytes = index_buffer.element_size()
+    res = C.c_void_p()
+    rep = report if report is not None else RsxReport()
+    with torch.cuda.device(src.device if src.is_cuda else None):
+        st = _lib().rsx_sort_rank_segments(src.data_ptr(), index_buffer.data_ptr(), n, off, nseg, C.byref(L), ib_bytes,
+                                           C.byref(res), C.byref(rep), _stream_ptr(src))
+    if st != RSX_OK:
+        raise RsxError(st, "rsx_sort_rank_segments")
+    off_el = (res.value - index_buffer.data_ptr()) // ib_bytes if n else 0
+    return index_buffer.view(-1)[off_el:off_el + n]
 
 
 def histogram(src, kf: Optional[KeyFunc] = None):

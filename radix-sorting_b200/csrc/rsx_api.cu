@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <mutex>
+#include <vector>
 
 #include "rsx_scatter_dispatch.cuh"
 
@@ -1108,6 +1109,257 @@ int rsx_sort_rank(const void *src, void *index_buffer, size_t n, const rsx_layou
 		*result = hres;
 	}
 	return r;
+}
+
+// ---- segmented sort ------------------------------------------------------------------------------
+// Host plan: consecutive short segments are packed into groups that one CTA sorts (rsx_segments.cu);
+// longer segments go through sort_device / rank_device one by one.  The batch's pass table comes
+// from one pre-pass over all n records, so every group writes into the buffer the reference's
+// parity rule designates for the batch.
+
+// offsets[0] == 0, non-decreasing, offsets[nseg] == n.  *max_len: the longest segment.
+static int check_offsets(const uint64_t *off, size_t nseg, size_t n, size_t *max_len) {
+	if (off[0] != 0 || off[nseg] != n)
+		return RSX_ERR_INVALID;
+	size_t m = 0;
+	for (size_t s = 0; s < nseg; ++s) {
+		if (off[s + 1] < off[s])
+			return RSX_ERR_INVALID;
+		m = off[s + 1] - off[s] > m ? off[s + 1] - off[s] : m;
+	}
+	*max_len = m;
+	return RSX_OK;
+}
+
+static bool idx_fits(int idx_bytes, size_t max_len) {
+	return idx_bytes == 0 || idx_bytes == 8 || max_len == 0 || ((max_len - 1) >> (8 * idx_bytes)) == 0;
+}
+
+// A pointer the runtime cannot classify (no driver, no device) cannot be device memory.
+static bool is_device_memory(const void *p) {
+	cudaPointerAttributes a;
+	if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+		(void)cudaGetLastError();
+		return false;
+	}
+	return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
+
+// Grow-only pinned host memory of the calling thread: the device offsets are read back into it and
+// the group plan is built in it and uploaded with one copy.  The calls using it are synchronous.
+static int segment_host_buffer(size_t bytes, unsigned char **out) {
+	thread_local void *buf = nullptr;
+	thread_local size_t cap = 0;
+	if (cap < bytes) {
+		if (buf)
+			cudaFreeHost(buf);
+		buf = nullptr;
+		cap = 0;
+		CU(cudaHostAlloc(&buf, bytes, cudaHostAllocPortable));
+		cap = bytes;
+	}
+	*out = static_cast<unsigned char *>(buf);
+	return RSX_OK;
+}
+
+// One walk over the offsets.  A group closes when the next segment would overflow one CTA (`cap`
+// records) or when it holds kMaxGroupSegments segments; empty segments take no part.  tab receives
+// every group's segment starts and length (see SegGroup).
+static void plan_groups(const uint64_t *off, size_t nseg, size_t cap, uint32_t *tab, size_t *ntab,
+                        std::vector<SegGroup> &groups, std::vector<size_t> &large) {
+	SegGroup g{};
+	size_t t = 0;
+	auto close = [&]() {
+		if (g.nseg) {
+			tab[t++] = g.len;
+			groups.push_back(g);
+		}
+		g = SegGroup{};
+	};
+	for (size_t s = 0; s < nseg; ++s) {
+		const size_t len = off[s + 1] - off[s];
+		if (len == 0)
+			continue;
+		if (len > cap) {
+			close();
+			large.push_back(s);
+			continue;
+		}
+		if (g.len + len > cap || g.nseg == kMaxGroupSegments)
+			close();
+		if (g.nseg == 0) {
+			g.begin = off[s];
+			g.tab = (uint32_t)t;
+		}
+		tab[t++] = g.len;
+		g.len += (uint32_t)len;
+		++g.nseg;
+	}
+	close();
+	*ntab = t;
+}
+
+static int sort_segments_common(const void *src, void *aux, void *ib, int idx_bytes, size_t n, const uint64_t *offsets,
+                                size_t nseg, const rsx_layout *layout, void **result, rsx_report *rep, void *stream) {
+	const bool ranksort = idx_bytes != 0;
+	KeyDesc kd;
+	int r = check_layout(layout, &kd); // records the tile kernels move directly: 1, 2, 4, 8 or 16 bytes
+	if (r)
+		return r;
+	if (ranksort && !(idx_bytes == 1 || idx_bytes == 2 || idx_bytes == 4 || idx_bytes == 8))
+		return RSX_ERR_INVALID;
+	if (!result || !offsets || (n && (!src || !(ranksort ? ib : aux))) || (nseg == 0 && n > 0))
+		return RSX_ERR_INVALID;
+	const uint32_t rb = layout->record_bytes;
+	if (!ranksort && n >= 2) {
+		const unsigned char *a = static_cast<const unsigned char *>(src), *b = static_cast<const unsigned char *>(aux);
+		if (a < b + n * rb && b < a + n * rb)
+			return RSX_ERR_INVALID;
+	}
+	// host offsets: everything is checked before any device work
+	const bool dev_offsets = is_device_memory(offsets);
+	size_t max_len = 0;
+	if (!dev_offsets) {
+		if ((r = check_offsets(offsets, nseg, n, &max_len)))
+			return r;
+		if (!idx_fits(idx_bytes, max_len))
+			return RSX_ERR_IDX_RANGE;
+	}
+	if (n < 2) { // one segment of at most one record: what rsx_sort / rsx_sort_rank do
+		if (ranksort)
+			return rsx_sort_rank(src, ib, n, layout, idx_bytes, result, rep, stream);
+		*result = const_cast<void *>(src);
+		trivial_report(rep);
+		return RSX_OK;
+	}
+	int dev;
+	if ((r = current_device(&dev)))
+		return r;
+	PtrKind ks, kb;
+	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(ranksort ? ib : aux, &kb)))
+		return r;
+	if (ks != PK_DEVICE || kb != PK_DEVICE)
+		return RSX_ERR_MIXED_MEMORY;
+	cudaStream_t st = static_cast<cudaStream_t>(stream);
+	const unsigned long long l0 = g_launches.load();
+	const size_t off_bytes = (nseg + 1) * sizeof(uint64_t);
+
+	// ---- plan on the host ----
+	unsigned char *hbuf = nullptr;
+	const size_t rd_bytes = dev_offsets ? align_up(off_bytes, 256) : 0;
+	const size_t tab_cap = align_up(2 * nseg * sizeof(uint32_t), 256); // <= one start per segment + one end per group
+	if ((r = segment_host_buffer(rd_bytes + tab_cap + nseg * sizeof(SegGroup), &hbuf)))
+		return r;
+	const uint64_t *hoff = offsets;
+	if (dev_offsets) { // read back once
+		CU(cudaMemcpyAsync(hbuf, offsets, off_bytes, cudaMemcpyDeviceToHost, st));
+		CU(cudaStreamSynchronize(st));
+		hoff = reinterpret_cast<const uint64_t *>(hbuf);
+		if ((r = check_offsets(hoff, nseg, n, &max_len)))
+			return r;
+		if (!idx_fits(idx_bytes, max_len))
+			return RSX_ERR_IDX_RANGE;
+	}
+	uint32_t *tab = reinterpret_cast<uint32_t *>(hbuf + rd_bytes);
+	size_t ntab = 0;
+	std::vector<SegGroup> groups;
+	std::vector<size_t> large;
+	plan_groups(hoff, nseg, segment_group_capacity(rb, ranksort), tab, &ntab, groups, large);
+	// the plan travels as [segment starts | groups]
+	const size_t tab_bytes = align_up(ntab * sizeof(uint32_t), 16), grp_bytes = groups.size() * sizeof(SegGroup);
+	memcpy(hbuf + rd_bytes + tab_bytes, groups.data(), grp_bytes);
+
+	// ---- pre-pass + group kernel: two launches for any number of short segments ----
+	Ctl c;
+	{
+		const size_t off_head = 0, off_offs = align_up(sizeof(WsHead), 256);
+		const size_t off_plan = off_offs + (dev_offsets ? 0 : align_up(off_bytes, 256));
+		Lease L;
+		if ((r = acquire(L, dev, off_plan + tab_bytes + grp_bytes)))
+			return r;
+		L.enqueued(st);
+		unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
+		WsHead *ws = reinterpret_cast<WsHead *>(wsp + off_head);
+		const unsigned long long *d_off = reinterpret_cast<const unsigned long long *>(offsets);
+		CU(cudaMemsetAsync(ws, 0, kWsZeroBytes, st));
+		if (!dev_offsets) {
+			CU(cudaMemcpyAsync(wsp + off_offs, offsets, off_bytes, cudaMemcpyHostToDevice, st));
+			d_off = reinterpret_cast<const unsigned long long *>(wsp + off_offs);
+		}
+		if (!groups.empty())
+			CU(cudaMemcpyAsync(wsp + off_plan, tab, tab_bytes + grp_bytes, cudaMemcpyHostToDevice, st));
+		CU(launch_segment_prepass(src, n, rb, kd, d_off, nseg, ws, L.pinned, g_dev[dev].num_sms, st));
+		if (!groups.empty())
+			CU(launch_segment_groups(src, const_cast<void *>(src), aux, ib, idx_bytes, n, rb, kd,
+			                         reinterpret_cast<const SegGroup *>(wsp + off_plan + tab_bytes), groups.size(),
+			                         reinterpret_cast<const uint32_t *>(wsp + off_plan), &ws->ctl, st));
+		CU(cudaStreamSynchronize(st));
+		L.drained();
+		c = *L.pinned;
+	} // the workspace is free again for the long segments' own sorts
+
+	const bool early = c.early_exit != 0, odd = !early && (c.ncols & 1u);
+	// ---- long segments: the ordinary path on the sub-range, result moved where the batch's lies ----
+	if (!large.empty() && !(early && !ranksort)) {
+		StageLease SL;
+		size_t max_large = 0;
+		for (size_t s : large)
+			max_large = hoff[s + 1] - hoff[s] > max_large ? hoff[s + 1] - hoff[s] : max_large;
+		if (ranksort) {
+			if ((r = acquire_stage(SL, dev, 2 * max_large * (size_t)idx_bytes)))
+				return r;
+			SL.inflight = st;
+			SL.has_inflight = true;
+		}
+		for (size_t s : large) {
+			const size_t o = hoff[s], len = hoff[s + 1] - o;
+			void *res = nullptr;
+			rsx_report srep;
+			if (ranksort) {
+				if ((r = rank_device(static_cast<const unsigned char *>(src) + o * rb, SL.ptr, len, layout, kd, idx_bytes, &res, &srep,
+				                     st, dev, false)))
+					return r;
+				unsigned char *to = static_cast<unsigned char *>(ib) + ((odd ? n : 0) + o) * (size_t)idx_bytes;
+				CU(cudaMemcpyAsync(to, res, len * (size_t)idx_bytes, cudaMemcpyDeviceToDevice, st));
+				CU(cudaStreamSynchronize(st)); // the staging buffer is reused by the next segment
+			} else {
+				unsigned char *s0 = static_cast<unsigned char *>(const_cast<void *>(src)) + o * rb;
+				unsigned char *a0 = static_cast<unsigned char *>(aux) + o * rb;
+				if ((r = sort_device(s0, a0, len, layout, kd, &res, &srep, st, dev, false)))
+					return r;
+				void *want = odd ? a0 : s0;
+				if (res != want)
+					CU(cudaMemcpyAsync(want, res, len * (size_t)rb, cudaMemcpyDeviceToDevice, st));
+			}
+		}
+		CU(cudaStreamSynchronize(st));
+		SL.has_inflight = false;
+	}
+	if (rep) {
+		memset(rep, 0, sizeof(*rep));
+		rep->early_exit = early;
+		rep->ncols = early ? 0 : c.ncols;
+		rep->live_mask = early ? 0 : c.live_mask;
+		rep->result_in_aux = odd;
+		rep->kernel_launches = (uint32_t)(g_launches.load() - l0);
+	}
+	if (ranksort)
+		*result = static_cast<unsigned char *>(ib) + (odd ? n * (size_t)idx_bytes : 0);
+	else
+		*result = odd ? aux : const_cast<void *>(src);
+	return RSX_OK;
+}
+
+int rsx_sort_segments(void *src, void *aux, size_t n, const uint64_t *offsets, size_t nseg, const rsx_layout *layout,
+                      void **result, rsx_report *report, void *stream) {
+	return sort_segments_common(src, aux, nullptr, 0, n, offsets, nseg, layout, result, report, stream);
+}
+
+int rsx_sort_rank_segments(const void *src, void *index_buffer, size_t n, const uint64_t *offsets, size_t nseg,
+                           const rsx_layout *layout, int idx_bytes, void **result, rsx_report *report, void *stream) {
+	if (idx_bytes == 0)
+		return RSX_ERR_INVALID;
+	return sort_segments_common(src, nullptr, index_buffer, idx_bytes, n, offsets, nseg, layout, result, report, stream);
 }
 
 // ---- halves of the path, for parity tests and profiling ------------------------------------------

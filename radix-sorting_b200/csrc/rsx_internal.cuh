@@ -124,6 +124,24 @@ size_t small_sort_capacity(uint32_t record_bytes, bool ranksort);
 cudaError_t launch_small_sort(const void *src, void *out_even, void *out_odd, void *index_buffer, int idx_bytes,
                               size_t n, uint32_t record_bytes, const KeyDesc &kd, Ctl *ctl, cudaStream_t st);
 
+// segmented sort (rsx_segments.cu).  A group is a run of consecutive non-empty segments that one CTA
+// sorts: records [begin, begin + len) of the batch, nseg segments whose group-local starts are
+// segtab[tab .. tab + nseg) followed by len.
+constexpr uint32_t kMaxGroupSegments = 256; // the segment id is one 8-bit digit
+struct SegGroup {
+	unsigned long long begin;
+	uint32_t len, nseg, tab, pad;
+};
+size_t segment_group_capacity(uint32_t record_bytes, bool ranksort);
+// OR / NAND of the derived keys and the descents inside segments -> the batch pass table in ws->ctl
+// (and host_ctl); ws's zeroed head must be clear.  offsets: nseg + 1 DEVICE entries.
+cudaError_t launch_segment_prepass(const void *src, size_t n, uint32_t record_bytes, const KeyDesc &kd,
+                                   const unsigned long long *offsets, size_t nseg, WsHead *ws, Ctl *host_ctl,
+                                   int num_sms, cudaStream_t st);
+cudaError_t launch_segment_groups(const void *src, void *out_even, void *out_odd, void *index_buffer, int idx_bytes, size_t n,
+                                  uint32_t record_bytes, const KeyDesc &kd, const SegGroup *groups, size_t ngroups,
+                                  const uint32_t *segtab, const Ctl *ctl, cudaStream_t st);
+
 // rank-sort helpers
 cudaError_t launch_iota_if_early(void *index_buffer, int idx_bytes, size_t n, const Ctl *ctl,
                                  cudaStream_t st);

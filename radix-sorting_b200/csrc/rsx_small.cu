@@ -9,16 +9,15 @@
 // ticket / ballot ranking exactly like K3), and a final store into the buffer the reference's
 // parity rule designates.  Same device pass table (Ctl) as the big path, so the host side is
 // unchanged: one launch, one 40-byte read-back.
-#include "rsx_scatter.cuh"
+#include "rsx_cta.cuh"
 
 namespace rsx {
 
 namespace {
 
-constexpr int kSmallThreads = 1024;
-constexpr int kSmallWarps = kSmallThreads / 32;
-constexpr int kSmallItems = 16; // records per thread per pass, at most
-constexpr size_t kSmallBytes = 64 * 1024; // per ping-pong buffer (records + index lane)
+constexpr int kSmallThreads = kCtaThreads;
+constexpr int kSmallWarps = kCtaWarps;
+constexpr size_t kSmallBytes = kCtaBufBytes; // per ping-pong buffer (records + index lane)
 
 struct SmallParams {
 	const void *src;      // input records
@@ -31,19 +30,9 @@ struct SmallParams {
 	Ctl *ctl;
 };
 
-template <typename T> __device__ __forceinline__ void store_index(void *ib, uint32_t idx_bytes, size_t at, T v) {
-	switch (idx_bytes) {
-	case 1: static_cast<uint8_t *>(ib)[at] = (uint8_t)v; break;
-	case 2: static_cast<uint16_t *>(ib)[at] = (uint16_t)v; break;
-	case 4: static_cast<uint32_t *>(ib)[at] = (uint32_t)v; break;
-	default: static_cast<unsigned long long *>(ib)[at] = (unsigned long long)v; break;
-	}
-}
-
 template <int ES, bool RANKSORT, int RANK>
 __global__ void __launch_bounds__(kSmallThreads, 1) small_sort_kernel(const SmallParams p) {
 	using R = typename Rec<ES>::type;
-	constexpr uint32_t FULL = 0xFFFFFFFFu;
 	constexpr uint32_t kCap = (uint32_t)((kSmallBytes - 16) / (ES + (RANKSORT ? 4 : 0)));
 	constexpr size_t kIdxOff = ((size_t)kCap * ES + 15) & ~(size_t)15; // index lane behind the records
 	extern __shared__ __align__(16) unsigned char smem[];
@@ -54,8 +43,7 @@ __global__ void __launch_bounds__(kSmallThreads, 1) small_sort_kernel(const Smal
 	uint32_t *s_hist = s_wh + kSmallWarps * kBins;                                  // [8 columns][256]
 	uint32_t *s_misc = s_hist + kMaxCols * kBins;                                   // scan scratch, live flags
 
-	const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
-	const uint32_t lt = lanemask_lt();
+	const uint32_t tid = threadIdx.x;
 	const uint32_t n = p.n;
 	const KeyDesc kd = p.kd;
 	const R *in = static_cast<const R *>(p.src);
@@ -100,89 +88,19 @@ __global__ void __launch_bounds__(kSmallThreads, 1) small_sort_kernel(const Smal
 	}
 	__syncthreads();
 
-	// each warp owns one contiguous chunk of the array (item i of lane l = chunk start + i*32 + l);
-	// only as many warps as the input needs take part in the per-warp prefix loops
-	constexpr uint32_t chunk = kSmallItems * 32;
-	const uint32_t nwarps = (n + chunk - 1) / chunk;
-	const uint32_t w0 = warp * chunk;
-	const uint32_t wend = min(n, w0 + chunk);
-	uint32_t *wh = s_wh + warp * kBins;
 	uint32_t cur = 0, ncols = 0, live_mask = 0;
 
 	for (uint32_t c = 0; c < kd.key_bytes; ++c) {
 		if (!s_misc[16 + c])
 			continue; // trivial column (uniform)
-		if (warp < nwarps)
-			for (uint32_t b = lane; b < kBins; b += 32)
-				wh[b] = 0;
-		__syncwarp();
-		// rank inside the warp, stable (items ascending, lanes ascending)
-		uint32_t rank[kSmallItems];
-#pragma unroll
-		for (int i = 0; i < kSmallItems; ++i) {
-			const uint32_t at = w0 + i * 32 + lane;
-			const bool valid = at < wend;
-			uint32_t d = 0;
-			if (valid)
-				d = (uint32_t)(derive_key(key_word<ES>(buf[cur][at], kd.word_sel), kd) >> (8 * c)) & 0xFFu;
-			if constexpr (RANK == RANK_TICKET) {
-				rank[i] = valid ? atomicAdd(&wh[d], 1u) : 0u;
-			} else {
-				uint32_t peers = __ballot_sync(FULL, valid);
-#pragma unroll
-				for (int b = 0; b < 8; ++b) {
-					const bool bit = (d >> b) & 1u;
-					const uint32_t v = __ballot_sync(FULL, bit);
-					peers &= bit ? v : ~v;
-				}
-				uint32_t old = 0;
-				const uint32_t leader = __ffs(peers) - 1;
-				if (valid && lane == leader)
-					old = atomicAdd(&wh[d], (uint32_t)__popc(peers));
-				old = __shfl_sync(FULL, old, valid ? leader : lane);
-				rank[i] = old + __popc(peers & lt);
-			}
-		}
-		__syncthreads();
-		// digit threads: prefix over the warps, exclusive scan over the digits
-		if (tid < kBins) {
-			uint32_t total = 0;
-			for (uint32_t w = 0; w < nwarps; ++w)
-				total += s_wh[w * kBins + tid];
-			uint32_t x = total;
-#pragma unroll
-			for (int o = 1; o < 32; o <<= 1) {
-				const uint32_t y = __shfl_up_sync(FULL, x, o);
-				if (lane >= o)
-					x += y;
-			}
-			if (lane == 31)
-				s_misc[warp] = x;
-			asm volatile("bar.sync 1, 256;" ::: "memory");
-			uint32_t run = x - total;
-			for (uint32_t w = 0; w < warp; ++w)
-				run += s_misc[w];
-			for (uint32_t w = 0; w < nwarps; ++w) {
-				const uint32_t cnt = s_wh[w * kBins + tid];
-				s_wh[w * kBins + tid] = run;
-				run += cnt;
-			}
-		}
-		__syncthreads();
-		// place (radix_sort.hpp:83-88)
-#pragma unroll
-		for (int i = 0; i < kSmallItems; ++i) {
-			const uint32_t at = w0 + i * 32 + lane;
-			if (at < wend) {
-				const R r = buf[cur][at];
-				const uint32_t d = (uint32_t)(derive_key(key_word<ES>(r, kd.word_sel), kd) >> (8 * c)) & 0xFFu;
-				const uint32_t pos = wh[d] + rank[i];
-				buf[cur ^ 1][pos] = r;
-				if constexpr (RANKSORT)
-					idx[cur ^ 1][pos] = idx[cur][at];
-			}
-		}
-		__syncthreads();
+		const auto digit = [&](const R &r, uint32_t) {
+			return (uint32_t)(derive_key(key_word<ES>(r, kd.word_sel), kd) >> (8 * c)) & 0xFFu;
+		};
+		R *const r0 = cur ? buf[1] : buf[0], *const r1 = cur ? buf[0] : buf[1];
+		if constexpr (RANKSORT)
+			cta_pass<ES, RANK>(r0, r1, cur ? idx[1] : idx[0], cur ? idx[0] : idx[1], n, s_wh, s_misc, digit);
+		else
+			cta_pass<ES, RANK, void>(r0, r1, nullptr, nullptr, n, s_wh, s_misc, digit);
 		cur ^= 1; // swap(src, aux), radix_sort.hpp:89
 		++ncols;
 		live_mask |= 1u << c;
@@ -227,7 +145,7 @@ cudaError_t launch_small_t(const SmallParams &sp, cudaStream_t st) {
 
 size_t small_sort_capacity(uint32_t record_bytes, bool ranksort) {
 	size_t cap = (kSmallBytes - 16) / (record_bytes + (ranksort ? 4 : 0));
-	const size_t by_items = (size_t)kSmallWarps * 32 * kSmallItems; // 16 records per thread
+	const size_t by_items = (size_t)kSmallWarps * 32 * kCtaItems; // 16 records per thread
 	return cap < by_items ? cap : by_items;
 }
 
