@@ -320,9 +320,9 @@ int rsx_version(void);
 uint64_t rsx_total_kernel_launches(void); /* process-wide count, for bench.py's gpu_launches */
 /* Options: "rank_mode" (-1 auto [default]: per-device hardware probe picks the one-instruction
  * ticket ranking or the ballot ranking, 0 force ticket, 1 force ballot; DESIGN.md "K3");
- * "query_rank_mode" returns the mode in effect (0 / 1).  "scatter_variant" (0..5) selects a tile
- * geometry used in tuning sweeps, "force_wide" (0/1) runs the n >= 2^30 (64-bit offset) kernels
- * at any n (tests).  "compact_min_n": key compaction is considered for keys-only sorts of at least
+ * "query_rank_mode" returns the mode in effect (0 / 1).  "scatter_variant" accepts only 0 (the
+ * shipped kernel choice) and changes nothing; any other value is RSX_ERR_INVALID.  "force_wide"
+ * (0/1) runs the n >= 2^30 (64-bit offset) kernels at any n (tests).  "compact_min_n": key compaction is considered for keys-only sorts of at least
  * this many 4/8-byte keys (default 2^26: below that the extra stream wait costs more than compaction can save; <= 0 disables it).  "profile" (0/1): bracket every kernel of rsx_sort / rsx_sort_rank with CUDA events on
  * the launch stream so that per-kernel device times can be read back with rsx_get_profile
  * (bench.py's roofline leg; off by default because the extra events perturb nothing but are

@@ -434,15 +434,6 @@ void trivial_report(rsx_report *rep) {
 
 } // namespace
 
-// RSX_SCATTER_VARIANT=<v> in the environment preselects a tuning variant (test runs under a variant)
-static int variant_from_env() {
-	const char *e = getenv("RSX_SCATTER_VARIANT");
-	const int v = e ? atoi(e) : 0;
-	return (v >= 0 && (v < kNumVariants || variant_is_v2(v))) ? v : 0;
-}
-static std::atomic<int> g_variant{variant_from_env()};
-int scatter_variant() { return g_variant.load(std::memory_order_relaxed); }
-
 int rank_mode() {
 	const int o = g_rank_override.load(std::memory_order_relaxed);
 	if (o == RANK_TICKET || o == RANK_BALLOT)
@@ -454,48 +445,43 @@ int rank_mode() {
 }
 
 // ---- launch glue declared in rsx_internal.cuh --------------------------------------------------
+template <class Cfg> void take_smaller_tile(PassGeometry &g, size_t smem) {
+	if (g.tile == 0 || Cfg::kThreads * Cfg::kItems < g.tile)
+		g = PassGeometry{Cfg::kThreads, Cfg::kItems, Cfg::kThreads * Cfg::kItems, smem, 0};
+}
 // Tile geometry that sizes the look-back state: the smallest tile any kernel of this footprint may
-// run with (the fused geometry, or a smaller tuning variant), so every kernel uses at most this
-// many status rows.
-PassGeometry scatter_geometry(uint32_t record_bytes, int payload_bytes) {
+// run with (the fused geometry, or the register-resident one), so every kernel uses at most this
+// many status rows.  Rank sorts of 1- and 2-byte keys through 32-bit index lanes reserve the rows of
+// a u32 rank sort, so their rsx_workspace_bytes stays what callers have been reserving.
+template <int ES, int PL> PassGeometry footprint_geometry() {
+	static_assert(FusedCfg<ES, PL>::kThreads * FusedCfg<ES, PL>::kItems <=
+	              ScatterCfg<ES, PL>::kThreads * ScatterCfg<ES, PL>::kItems, "fused tile must be the smallest");
 	PassGeometry g{};
-	const int v = scatter_variant();
-	auto take = [&](uint32_t threads, uint32_t items, size_t smem) {
-		if (g.threads == 0 || threads * items < g.threads * g.items) {
-			g.threads = threads;
-			g.items = items;
-			g.smem_bytes = smem;
-		}
-	};
-#define GEOV(ES, PL, V)                                                                          \
-	if (record_bytes == ES && payload_bytes == PL && v == V)                                     \
-		take(ScatterCfgV<ES, PL, V>::kThreads, ScatterCfgV<ES, PL, V>::kItems,                   \
-		     ScatterSmem<ES, PL, ScatterCfgV<ES, PL, V>, false>::kBytes);
-#define GEO2V(ES, PL, V)                                                                         \
-	if (record_bytes == ES && payload_bytes == PL && v == kVariant2Base + V)                     \
-		take(Cfg2V<ES, PL, V>::kThreads, Cfg2V<ES, PL, V>::kItems, Scatter2Smem<ES, PL, Cfg2V<ES, PL, V>>::kBytes);
-#define GEO(ES, PL)                                                                              \
-	if (record_bytes == ES && payload_bytes == PL) {                                             \
-		static_assert(FusedCfg<ES, PL>::kThreads * FusedCfg<ES, PL>::kItems <=                   \
-		              ScatterCfg<ES, PL>::kThreads * ScatterCfg<ES, PL>::kItems, "fused tile must be the smallest"); \
-		take(FusedCfg<ES, PL>::kThreads, FusedCfg<ES, PL>::kItems, ScatterSmem<ES, PL, FusedCfg<ES, PL>, true>::kBytes); \
-		/* the register-resident kernel's default geometry (PreferV2 or variant 10) */            \
-		take(Cfg2V<ES, PL, 0>::kThreads, Cfg2V<ES, PL, 0>::kItems, Scatter2Smem<ES, PL, Cfg2V<ES, PL, 0>>::kBytes); \
-	}
-	GEO(1, 0) GEO(1, 4) GEO(1, 8) GEO(2, 0) GEO(2, 4) GEO(2, 8) GEO(4, 0) GEO(4, 4) GEO(4, 8)
-	GEO(8, 0) GEO(8, 4) GEO(8, 8) GEO(16, 0) GEO(16, 4) GEO(16, 8)
-	GEOV(4, 0, 1) GEOV(4, 0, 2) GEOV(4, 0, 3) GEOV(4, 0, 4) GEOV(4, 0, 5) GEOV(4, 0, 6) GEOV(4, 0, 7) GEOV(4, 0, 8) GEOV(4, 0, 9)
-	GEOV(8, 0, 1) GEOV(8, 0, 2) GEOV(8, 0, 3) GEOV(8, 0, 4) GEOV(8, 0, 5) GEOV(8, 0, 6) GEOV(8, 0, 7) GEOV(8, 0, 8) GEOV(8, 0, 9)
-	GEO2V(4, 0, 1) GEO2V(4, 0, 2) GEO2V(4, 0, 3) GEO2V(4, 0, 4) GEO2V(4, 0, 5) GEO2V(4, 0, 6) GEO2V(4, 0, 7) GEO2V(4, 0, 8) GEO2V(4, 0, 9)
-	GEO2V(4, 0, 10) GEO2V(4, 0, 11) GEO2V(4, 0, 12) GEO2V(4, 0, 13) GEO2V(4, 0, 14) GEO2V(4, 0, 15) GEO2V(4, 0, 16) GEO2V(4, 0, 17) GEO2V(4, 0, 18) GEO2V(4, 0, 19) GEO2V(4, 0, 20) GEO2V(4, 0, 21) GEO2V(4, 0, 22) GEO2V(4, 0, 23)
-	GEO2V(8, 0, 1) GEO2V(8, 0, 2) GEO2V(8, 0, 3) GEO2V(8, 0, 4) GEO2V(8, 0, 5) GEO2V(8, 0, 6) GEO2V(8, 0, 7) GEO2V(8, 0, 8) GEO2V(8, 0, 9)
-	GEO2V(8, 0, 10) GEO2V(8, 0, 11) GEO2V(8, 0, 12) GEO2V(8, 0, 13) GEO2V(8, 0, 14) GEO2V(8, 0, 15) GEO2V(8, 0, 16) GEO2V(8, 0, 17) GEO2V(8, 0, 18) GEO2V(8, 0, 19) GEO2V(8, 0, 20) GEO2V(8, 0, 21) GEO2V(8, 0, 22) GEO2V(8, 0, 23)
-#undef GEO2V
-#undef GEO
-#undef GEOV
-	g.tile = g.threads * g.items;
-	g.ctas_per_sm = 0;
+	take_smaller_tile<FusedCfg<ES, PL>>(g, ScatterSmem<ES, PL, FusedCfg<ES, PL>, true>::kBytes);
+	if constexpr (PreferV2<ES, PL>::value)
+		take_smaller_tile<Cfg2<ES, PL>>(g, Scatter2Smem<ES, PL, Cfg2<ES, PL>>::kBytes);
+	else if constexpr (ES < 4 && PL == 4)
+		take_smaller_tile<Cfg2<4, 4>>(g, Scatter2Smem<ES, PL, Cfg2<4, 4>>::kBytes);
 	return g;
+}
+template <int ES> PassGeometry footprint_geometry(int payload_bytes) {
+	switch (payload_bytes) {
+	case 0: return footprint_geometry<ES, 0>();
+	case 4: return footprint_geometry<ES, 4>();
+	case 8: return footprint_geometry<ES, 8>();
+	}
+	return PassGeometry{};
+}
+
+PassGeometry scatter_geometry(uint32_t record_bytes, int payload_bytes) {
+	switch (record_bytes) {
+	case 1: return footprint_geometry<1>(payload_bytes);
+	case 2: return footprint_geometry<2>(payload_bytes);
+	case 4: return footprint_geometry<4>(payload_bytes);
+	case 8: return footprint_geometry<8>(payload_bytes);
+	case 16: return footprint_geometry<16>(payload_bytes);
+	}
+	return PassGeometry{};
 }
 
 cudaError_t launch_scatter(const PassBuffers &pb, size_t n, uint32_t record_bytes, int payload_bytes,
@@ -605,12 +591,8 @@ int rsx_set_option(const char *name, long value) {
 		g_rank_override.store((int)value);
 		return RSX_OK;
 	}
-	if (name && strcmp(name, "scatter_variant") == 0) { // tuning experiments, see rsx_scatter.cuh
-		if (value < 0 || (value >= kNumVariants && !variant_is_v2((int)value)))
-			return RSX_ERR_INVALID;
-		g_variant.store((int)value);
-		return RSX_OK;
-	}
+	if (name && strcmp(name, "scatter_variant") == 0) // only the default kernel choice exists
+		return value == 0 ? RSX_OK : RSX_ERR_INVALID;
 	if (name && strcmp(name, "small_path") == 0) { // 0: always use the multi-kernel path (tests)
 		g_small_path.store(value ? 1 : 0);
 		return RSX_OK;

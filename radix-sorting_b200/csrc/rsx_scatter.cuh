@@ -181,47 +181,12 @@ template <int ES> __device__ __forceinline__ typename Rec<ES>::type make_pad(con
 		return (typename Rec<ES>::type)p.x;
 }
 
-// Tile geometry per (record, payload) footprint.  kStage: the next tile is prefetched by a TMA
-// bulk copy into a staging buffer while the current tile is ranked / scattered / stored.
-// V selects a tuning variant (rsx_set_option("scatter_variant", V)); V = 0 is the default.
-// MD (ticket ranking only):
-//   0  rank = ticket atomic in the ranking sweep, kept (two per register) until the placement looks
-//      the warp's bucket base up:                                   1 ATOMS + 1 LDS per record
-//   1  the first sweep only counts; once the digit scan has turned the warp counters into slot
-//      bases the placement sweep takes its slot with the ticket atomic itself (same sweep order,
-//      hence the same stable order):                                2 ATOMS per record, no rank registers
-// ELB: the first look-back window is LOADED before the placement sweep and evaluated after it, so
-//      its L2 round trip overlaps the placement instead of following it.
-// SLB: split look-back -- the digit threads (warps 0-7) walk the look-back chain right after the
-//      digit scan, WHILE warps 8.. place their records, and place their own afterwards: the chain's
-//      L2 round trips overlap the placement, and this tile's inclusive prefix is published one
-//      placement phase earlier (which shortens every successor's chain).
-template <int T, int I, int MB, int LBK, bool ST, int MD = 0, bool ELB = false, bool SLB = false> struct CfgT {
-	static constexpr int kThreads = T, kItems = I, kMinBlocks = MB, kLookback = LBK, kMode = MD;
-	static constexpr bool kStage = ST, kEarlyLookback = ELB, kSplitLookback = SLB;
+// Tile geometry per (record, payload) footprint: threads, records per thread, minimum CTAs per SM
+// (launch bounds) and look-back window (status words per digit thread and round).
+template <int T, int I, int MB, int LBK> struct CfgT {
+	static constexpr int kThreads = T, kItems = I, kMinBlocks = MB, kLookback = LBK;
 };
 
-// Predicated shared-memory ticket: lanes with skip == true keep `r` (their vote-derived rank).
-// One predicated ATOMS instead of a divergent branch per item.
-__device__ __forceinline__ uint32_t ticket_unless(uint32_t *addr, bool skip, uint32_t r) {
-	asm volatile("{\n"
-	             ".reg .pred q;\n"
-	             "setp.eq.u32 q, %2, 0;\n"
-	             "@q atom.shared.add.u32 %0, [%1], 1;\n"
-	             "}\n"
-	             : "+r"(r)
-	             : "r"((uint32_t)__cvta_generic_to_shared(addr)), "r"((uint32_t)skip)
-	             : "memory");
-	return r;
-}
-__device__ __forceinline__ void count_unless(uint32_t *addr, bool skip) {
-	asm volatile("{\n"
-	             ".reg .pred q;\n"
-	             "setp.eq.u32 q, %1, 0;\n"
-	             "@q red.shared.add.u32 [%0], 1;\n"
-	             "}\n" ::"r"((uint32_t)__cvta_generic_to_shared(addr)), "r"((uint32_t)skip)
-	             : "memory");
-}
 // Defaults from the B200 sweeps recorded in profiles/r1_variants.md.  The pass is bound by the
 // shared-memory/LSU data pipe and by per-tile fixed costs (barriers, look-back), so the tile is as
 // large as shared memory allows: 4-byte footprints run 512 threads x 22 records with two CTAs per
@@ -231,50 +196,25 @@ __device__ __forceinline__ void count_unless(uint32_t *addr, bool skip) {
 // Look-back window: every tile reads 2 x LB x 256 status words in its first round (32 KB at LB 16
 // against a 45 KB tile of 4-byte keys); 8 words per thread cost a few more serial rounds but 7 % less
 // time per u32 pass (LB 4 / 6 / 8 / 12 / 16: 2.59 / 2.58 / 2.59 / 2.67 / 2.79 ms).
-template <int ES, int PL, int V> struct ScatterCfgV
-	: CfgT<512, ((ES + PL <= 4) ? 22 : 192 / (ES + PL)), ((ES + PL <= 4) ? 2 : 1), 8, true> {};
+template <int ES, int PL> struct ScatterCfg
+	: CfgT<512, ((ES + PL <= 4) ? 22 : 192 / (ES + PL)), ((ES + PL <= 4) ? 2 : 1), 8> {};
 // The fused partition + exchange passes (multi-GPU) carry a 4 KB destination table in shared
 // memory and keep the geometry they were tuned and measured with.  It is the smallest tile of any
 // default kernel, so it also sizes the look-back state (scatter_geometry()).
 template <int ES, int PL> struct FusedCfg
 	: CfgT<((ES + PL > 4 && ES + PL <= 8) ? 1024 : 512),
 	       ((ES + PL <= 4) ? 20 : (ES + PL <= 8) ? 10 : (ES + PL <= 16) ? 8 : 4), ((ES + PL <= 4) ? 2 : 1),
-	       ((ES + PL <= 4) ? 8 : 16), true> {};
-constexpr int kNumVariants = 10;
-// Tuning variants (bench.py --variant V, tools/gpu_ab.sh) exist for plain 4- and 8-byte keys only:
-// the neighbours of the default in the last sweep (profiles/r1_variants.md, "Final geometry"),
-// V = 2 being the geometry most of round 1 was measured with.
-template <> struct ScatterCfgV<4, 0, 1> : CfgT<256, 44, 2, 8, true> {};
-template <> struct ScatterCfgV<4, 0, 2> : CfgT<384, 29, 2, 8, true> {};
-template <> struct ScatterCfgV<4, 0, 3> : CfgT<256, 44, 2, 16, true> {};
-template <> struct ScatterCfgV<4, 0, 4> : CfgT<512, 40, 1, 8, true> {};
-template <> struct ScatterCfgV<4, 0, 5> : CfgT<512, 44, 1, 8, true> {};
-template <> struct ScatterCfgV<4, 0, 6> : CfgT<512, 22, 2, 8, true, 0, true> {};
-template <> struct ScatterCfgV<4, 0, 7> : CfgT<512, 22, 2, 8, true, 1, false> {};
-template <> struct ScatterCfgV<4, 0, 8> : CfgT<512, 22, 2, 8, true, 0, false, true> {};
-template <> struct ScatterCfgV<4, 0, 9> : CfgT<512, 22, 2, 16, true, 0, false, true> {};
-template <> struct ScatterCfgV<8, 0, 6> : CfgT<512, 24, 1, 8, true, 0, true> {};
-template <> struct ScatterCfgV<8, 0, 7> : CfgT<512, 24, 1, 8, true, 1, false> {};
-template <> struct ScatterCfgV<8, 0, 8> : CfgT<512, 24, 1, 8, true, 0, false, true> {};
-template <> struct ScatterCfgV<8, 0, 9> : CfgT<512, 24, 1, 16, true, 0, false, true> {};
-template <> struct ScatterCfgV<8, 0, 1> : CfgT<256, 24, 2, 8, true> {};
-template <> struct ScatterCfgV<8, 0, 2> : CfgT<384, 16, 2, 8, true> {};
-template <> struct ScatterCfgV<8, 0, 3> : CfgT<256, 24, 2, 16, true> {};
-template <> struct ScatterCfgV<8, 0, 4> : CfgT<256, 48, 1, 8, true> {};
-template <> struct ScatterCfgV<8, 0, 5> : CfgT<384, 32, 1, 8, true> {};
-template <int ES, int PL> using ScatterCfg = ScatterCfgV<ES, PL, 0>;
-int scatter_variant();
+	       ((ES + PL <= 4) ? 8 : 16)> {};
 
 template <int ES, int PL, class Cfg, bool FUSED = true> struct ScatterSmem {
 	static constexpr int kTile = Cfg::kThreads * Cfg::kItems;
 	static constexpr int kWarps = Cfg::kThreads / 32;
 	static constexpr size_t kRecBytes = (size_t)kTile * ES;
 	static constexpr size_t kPlBytes = (size_t)kTile * PL;
-	static constexpr size_t kStageBytes = kRecBytes + kPlBytes;
 	static constexpr size_t kWhBytes = (size_t)kWarps * kBins * 4;
 	static constexpr size_t kAdjBytes = (size_t)kBins * 8;
 	// layout: [stage rec | stage pl | sorted rec | sorted pl | warp counters | gadj | misc]
-	static constexpr size_t kOffSorted = kStageBytes;
+	static constexpr size_t kOffSorted = kRecBytes + kPlBytes; // after the staging buffer
 	static constexpr size_t kSortedSlack = 0; // fused mode may read one 16-byte vector past the sorted buffer: that is the counter area, harmless
 	static constexpr size_t kOffWh = kOffSorted + kRecBytes + kSortedSlack + kPlBytes;
 	static constexpr size_t kOffAdj = kOffWh + kWhBytes;
@@ -296,11 +236,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 	constexpr int TILE = SM::kTile;
 	constexpr int WARPS = SM::kWarps;
 	constexpr int LB = Cfg::kLookback;
-#ifdef RSX_WRITE_BATCH
-	constexpr int kWriteBatch = RSX_WRITE_BATCH;
-#else
-	constexpr int kWriteBatch = 2;
-#endif
+	constexpr int kWriteBatch = 2; // records per write-out batch (see step 5)
 	constexpr uint32_t FULL = 0xFFFFFFFFu;
 	static_assert(THREADS >= kBins && THREADS % 32 == 0, "one digit thread per bin: the digit scan synchronises 256 threads");
 
@@ -417,52 +353,23 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 		RSX_T(0);
 
 		// ---- 2. rank inside the warp (stable: items ascending, lanes ascending) ----
-		constexpr int MODE = RANK == RANK_TICKET ? Cfg::kMode : 0;
-		// Ranks are packed two per register only where the registers are needed for the early
-		// look-back window; unpacked ranks + a branch around the atomic measured 1-2 % faster on
-		// uniform digits (profiles/r2_variants.md).
-		constexpr bool PACK = Cfg::kEarlyLookback;
-		uint32_t rank[MODE != 0 ? 1 : PACK ? (ITEMS + 1) / 2 : ITEMS];
-		auto set_rank = [&](int i, uint32_t r) {
-			if constexpr (!PACK)
-				rank[i] = r;
-			else if (i & 1)
-				rank[i >> 1] |= r << 16;
-			else
-				rank[i >> 1] = r;
-		};
-		auto get_rank = [&](int i) -> uint32_t {
-			if constexpr (!PACK)
-				return rank[i];
-			else
-				return (i & 1) ? (rank[i >> 1] >> 16) : (rank[i >> 1] & 0xFFFFu);
-		};
-		[[maybe_unused]] uint32_t hot = 0;
+		uint32_t rank[ITEMS];
 		if constexpr (RANK == RANK_TICKET) {
 			// The tile's most frequent digit of the previous tile ("hot") is ranked in registers:
 			// one vote per item instead of up to 32 same-address atomics when a digit dominates
 			// (low-entropy columns); for uniform digits it only removes a few lanes from the atomic.
-			hot = s_misc[9];
+			const uint32_t hot = s_misc[9];
 			uint32_t hotcnt = 0;
 #pragma unroll
 			for (int i = 0; i < ITEMS; ++i) { // fully unrolled on purpose (partial: +8 %)
 				const uint32_t d = tile_digit<ES, DM>(p, s_stage[t0 + i * 32], dd);
 				const bool is_hot = d == hot;
 				const uint32_t m = __ballot_sync(FULL, is_hot);
-				if constexpr (MODE == 0) {
-					if constexpr (!PACK) {
-						uint32_t r; // a branch, not a predicated atomic: 1-2 % faster on uniform digits
-						if (is_hot)
-							r = hotcnt + __popc(m & lt);
-						else
-							r = atomicAdd(&wh[d], 1u);
-						set_rank(i, r);
-					} else {
-						set_rank(i, ticket_unless(&wh[d], is_hot, hotcnt + __popc(m & lt)));
-					}
-				} else {
-					count_unless(&wh[d], is_hot);
-				}
+				// a branch, not a predicated atomic: 1-2 % faster on uniform digits (profiles/r2_variants.md)
+				if (is_hot)
+					rank[i] = hotcnt + __popc(m & lt);
+				else
+					rank[i] = atomicAdd(&wh[d], 1u);
 				hotcnt += __popc(m);
 			}
 			if (lane == 0)
@@ -483,7 +390,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 				if (lane == leader)
 					old = atomicAdd(&wh[d], (uint32_t)__popc(peers));
 				old = __shfl_sync(FULL, old, leader);
-				set_rank(i, old + __popc(peers & lt));
+				rank[i] = old + __popc(peers & lt);
 			}
 		}
 		RSX_T(1);
@@ -584,57 +491,27 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 		__syncthreads(); // (C)
 		RSX_T(4);
 
-		// ---- (3b, early) first look-back window: loads issued now, evaluated after the placement ----
-		constexpr bool SLB = Cfg::kSplitLookback && THREADS >= 2 * kBins;
-		constexpr bool kPair = THREADS >= 2 * kBins && !SLB;
-		constexpr bool ELB = Cfg::kEarlyLookback && !SLB;
-		const uint32_t dgt = tid & (kBins - 1), half = tid / kBins;
-		[[maybe_unused]] OffT lbw[LB];
-		if constexpr (ELB) {
-			if (half < (kPair ? 2u : 1u)) {
-				const int q = (int)tile - 1 - (int)half * LB;
-#pragma unroll
-				for (int j = 0; j < LB; ++j)
-					lbw[j] = (q - j >= 0) ? ld_status(&status[(size_t)(q - j) * kBins + dgt]) : (OffT)SB::kPfx;
-			}
-		}
-
-		// ---- 4. records / payloads to their tile-sorted slot ----
+		// ---- 4. records / payloads to their tile-sorted slot.  (A lambda called once: written
+		//      inline, the compiler hoists the warp-counter address differently and allocates
+		//      registers differently for the whole kernel.) ----
 		auto place = [&]() {
-			if constexpr (MODE == 0) {
 #pragma unroll
-				for (int i = 0; i < ITEMS; ++i) { // fully unrolled on purpose: partial unrolling costs 10 %
-					const R r = s_stage[t0 + i * 32];
-					const uint32_t pos = wh[tile_digit<ES, DM>(p, r, dd)] + get_rank(i);
-					s_rec[pos] = r;
-					if constexpr (PL != 0)
-						s_pl[pos] = synth ? (P)(base + t0 + i * 32) : s_stage_pl[t0 + i * 32];
-				}
-			} else {
-				// same sweep order as the count: the ticket now returns the slot itself
-				uint32_t hotpos = wh[hot];
-				__syncwarp();
-#pragma unroll
-				for (int i = 0; i < ITEMS; ++i) {
-					const R r = s_stage[t0 + i * 32];
-					const uint32_t d = tile_digit<ES, DM>(p, r, dd);
-					const bool is_hot = d == hot;
-					const uint32_t m = __ballot_sync(FULL, is_hot);
-					const uint32_t pos = ticket_unless(&wh[d], is_hot, hotpos + __popc(m & lt));
-					hotpos += __popc(m);
-					s_rec[pos] = r;
-					if constexpr (PL != 0)
-						s_pl[pos] = synth ? (P)(base + t0 + i * 32) : s_stage_pl[t0 + i * 32];
-				}
+			for (int i = 0; i < ITEMS; ++i) { // fully unrolled on purpose: partial unrolling costs 10 %
+				const R r = s_stage[t0 + i * 32];
+				const uint32_t pos = wh[tile_digit<ES, DM>(p, r, dd)] + rank[i];
+				s_rec[pos] = r;
+				if constexpr (PL != 0)
+					s_pl[pos] = synth ? (P)(base + t0 + i * 32) : s_stage_pl[t0 + i * 32];
 			}
 		};
-		if (!SLB || tid >= kBins)
-			place();
+		place();
 		RSX_T(5);
 
 		// ---- 3b. decoupled look-back, one chain per digit.  The first round is split over two
 		//      threads per digit (warp w and warp w+8), so 2*LB predecessors cost one L2 round trip;
 		//      whatever is still unresolved afterwards is walked serially by the digit thread. ----
+		constexpr bool kPair = THREADS >= 2 * kBins;
+		const uint32_t dgt = tid & (kBins - 1), half = tid / kBins;
 		bool append_mode = false;
 		if constexpr (FUSED)
 			append_mode = p.dest_cursor != nullptr;
@@ -653,17 +530,11 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 			OffT part = 0;
 			uint32_t st = 0, used = 0; // st: 0 = only aggregates so far, 1 = reached a prefix, 2 = hit an unpublished word
 			if (half < (kPair ? 2u : 1u)) {
+				const int q = (int)tile - 1 - (int)half * LB;
 				OffT w[LB];
-				if constexpr (ELB) {
 #pragma unroll
-					for (int j = 0; j < LB; ++j)
-						w[j] = lbw[j];
-				} else {
-					const int q = (int)tile - 1 - (int)half * LB;
-#pragma unroll
-					for (int j = 0; j < LB; ++j)
-						w[j] = (q - j >= 0) ? ld_status(&status[(size_t)(q - j) * kBins + dgt]) : (OffT)SB::kPfx;
-				}
+				for (int j = 0; j < LB; ++j)
+					w[j] = (q - j >= 0) ? ld_status(&status[(size_t)(q - j) * kBins + dgt]) : (OffT)SB::kPfx;
 #pragma unroll
 				for (int j = 0; j < LB; ++j) {
 					if (st == 0) {
@@ -757,10 +628,6 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter_kernel
 					s_gadj[dgt] = (OffT)p.offs[dgt] + excl - (OffT)tstart;
 				}
 			}
-		}
-		if constexpr (SLB) {
-			if (tid < kBins)
-				place();
 		}
 		RSX_T(6);
 		if (tid == 0) // next ticket: claimed as late as possible (see above)

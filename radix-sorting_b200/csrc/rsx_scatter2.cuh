@@ -12,8 +12,10 @@
 //     tile drains to global memory -- the register file is the prefetch buffer;
 //   * a record is touched in shared memory exactly twice: the scatter into its tile-sorted slot
 //     and the linear read of the write-out;
-//   * the stable in-warp rank of two records is packed into one register between the ranking
-//     and the placement;
+//   * ranking only counts; once the digit scan has turned the warp counters into slot bases, the
+//     placement sweep takes each record's slot with the ticket atomic itself (same sweep order,
+//     hence the same stable order): 2 ATOMS per record and no rank registers, which leaves the
+//     register file to the tile;
 //   * shared memory per CTA is one sorted tile + the warp counters, so more CTAs (or larger
 //     tiles) fit per SM and the barrier / look-back bubbles of one CTA are filled by another.
 // Ranking is the one-instruction ticket (rank = atomicAdd(&warp_counter[digit], 1), see
@@ -25,14 +27,27 @@
 
 namespace rsx {
 
-// MODE 0: rank = ticket atomic during the ranking sweep, kept (two per register) until the
-//         placement looks the warp's bucket base up:          1 ATOMS + 1 LDS per record
-// MODE 1: the first sweep only counts (no return value, no rank registers); after the digit scan
-//         has turned the warp counters into slot bases the placement takes its slot with the
-//         ticket atomic itself:                                2 ATOMS per record, fewer registers
-template <int T, int I, int MB, int LBK, int MD = 0> struct Cfg2T {
-	static constexpr int kThreads = T, kItems = I, kMinBlocks = MB, kLookback = LBK, kMode = MD;
-};
+// Predicated shared-memory ticket: lanes with skip == true keep `r` (their vote-derived rank).
+// One predicated ATOMS instead of a divergent branch per item.
+__device__ __forceinline__ uint32_t ticket_unless(uint32_t *addr, bool skip, uint32_t r) {
+	asm volatile("{\n"
+	             ".reg .pred q;\n"
+	             "setp.eq.u32 q, %2, 0;\n"
+	             "@q atom.shared.add.u32 %0, [%1], 1;\n"
+	             "}\n"
+	             : "+r"(r)
+	             : "r"((uint32_t)__cvta_generic_to_shared(addr)), "r"((uint32_t)skip)
+	             : "memory");
+	return r;
+}
+__device__ __forceinline__ void count_unless(uint32_t *addr, bool skip) {
+	asm volatile("{\n"
+	             ".reg .pred q;\n"
+	             "setp.eq.u32 q, %1, 0;\n"
+	             "@q red.shared.add.u32 [%0], 1;\n"
+	             "}\n" ::"r"((uint32_t)__cvta_generic_to_shared(addr)), "r"((uint32_t)skip)
+	             : "memory");
+}
 
 template <int ES, int PL, class Cfg> struct Scatter2Smem {
 	static constexpr int kTile = Cfg::kThreads * Cfg::kItems;
@@ -48,74 +63,26 @@ template <int ES, int PL, class Cfg> struct Scatter2Smem {
 	static constexpr size_t kBytes = kOffMisc + 96;
 };
 
-// ---- tile geometry of the register-resident kernel ---------------------------------------------
-// V = 0 is the default per footprint (record + payload bytes); V >= 1 are tuning variants for plain
-// 4- and 8-byte keys (rsx_set_option("scatter_variant", 10 + V), tools/sweep_variants.py).
-template <int ES, int PL, int V> struct Cfg2V
-	: Cfg2T<((ES + PL > 4 && ES + PL <= 8) ? 256 : 512),
-	        ((ES + PL <= 4) ? 22 : (ES + PL <= 8) ? 32 : (ES + PL <= 16) ? 8 : 6), 2, 8, ((ES + PL > 4 && ES + PL <= 8) ? 1 : 0)> {};
-constexpr int kNumVariants2 = 24;
-// 8-byte keys: 36 records per thread measured 1.4 % faster than 32 (3.95 vs 4.01 ms per 1 B-key pass)
-template <> struct Cfg2V<8, 0, 0> : Cfg2T<256, 36, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 1> : Cfg2T<512, 20, 2, 8> {};
-template <> struct Cfg2V<4, 0, 2> : Cfg2T<384, 24, 2, 8> {};
-template <> struct Cfg2V<4, 0, 3> : Cfg2T<256, 22, 4, 8> {};
-template <> struct Cfg2V<4, 0, 4> : Cfg2T<256, 28, 3, 8> {};
-template <> struct Cfg2V<4, 0, 5> : Cfg2T<1024, 22, 1, 8> {};
-template <> struct Cfg2V<4, 0, 6> : Cfg2T<384, 16, 3, 8> {};
-template <> struct Cfg2V<4, 0, 7> : Cfg2T<384, 30, 2, 8> {};
-template <> struct Cfg2V<4, 0, 8> : Cfg2T<512, 22, 2, 4> {};
-template <> struct Cfg2V<4, 0, 9> : Cfg2T<512, 18, 2, 8> {};
-template <> struct Cfg2V<8, 0, 1> : Cfg2T<256, 24, 2, 8> {};
-template <> struct Cfg2V<8, 0, 2> : Cfg2T<384, 16, 2, 8> {};
-template <> struct Cfg2V<8, 0, 3> : Cfg2T<512, 24, 1, 8> {};
-template <> struct Cfg2V<8, 0, 4> : Cfg2T<256, 32, 2, 8> {};
-template <> struct Cfg2V<8, 0, 5> : Cfg2T<256, 40, 2, 8> {};
-template <> struct Cfg2V<8, 0, 6> : Cfg2T<256, 24, 3, 8> {};
-template <> struct Cfg2V<8, 0, 7> : Cfg2T<512, 14, 2, 8> {};
-template <> struct Cfg2V<8, 0, 8> : Cfg2T<1024, 12, 1, 8> {};
-template <> struct Cfg2V<8, 0, 9> : Cfg2T<512, 12, 2, 16> {};
-// 10..19: the count + ticket-placement form (MODE 1)
-template <> struct Cfg2V<4, 0, 10> : Cfg2T<512, 22, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 11> : Cfg2T<512, 26, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 12> : Cfg2T<384, 24, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 13> : Cfg2T<256, 22, 4, 8, 1> {};
-template <> struct Cfg2V<4, 0, 14> : Cfg2T<256, 28, 3, 8, 1> {};
-template <> struct Cfg2V<4, 0, 15> : Cfg2T<1024, 22, 1, 8, 1> {};
-template <> struct Cfg2V<4, 0, 16> : Cfg2T<384, 20, 3, 8, 1> {};
-template <> struct Cfg2V<4, 0, 17> : Cfg2T<384, 32, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 18> : Cfg2T<512, 30, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 19> : Cfg2T<640, 22, 1, 8, 1> {};
-// 20..23: few fat threads (the shape that won for 8-byte records), 4-byte keys
-template <> struct Cfg2V<4, 0, 20> : Cfg2T<256, 44, 2, 8, 1> {};
-template <> struct Cfg2V<4, 0, 21> : Cfg2T<256, 44, 3, 8, 1> {};
-template <> struct Cfg2V<4, 0, 22> : Cfg2T<256, 36, 3, 8, 1> {};
-template <> struct Cfg2V<4, 0, 23> : Cfg2T<256, 56, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 20> : Cfg2T<256, 28, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 21> : Cfg2T<256, 36, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 22> : Cfg2T<320, 26, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 23> : Cfg2T<256, 30, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 10> : Cfg2T<512, 12, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 11> : Cfg2T<512, 16, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 12> : Cfg2T<384, 20, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 13> : Cfg2T<512, 24, 1, 8, 1> {};
-template <> struct Cfg2V<8, 0, 14> : Cfg2T<256, 32, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 15> : Cfg2T<256, 40, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 16> : Cfg2T<256, 24, 3, 8, 1> {};
-template <> struct Cfg2V<8, 0, 17> : Cfg2T<512, 20, 2, 8, 1> {};
-template <> struct Cfg2V<8, 0, 18> : Cfg2T<1024, 12, 1, 8, 1> {};
-template <> struct Cfg2V<8, 0, 19> : Cfg2T<384, 24, 2, 8, 1> {};
-
-// Which kernel runs a single-GPU pass when no variant is forced: flipped per footprint by
-// measurement (profiles/r2_variants.md).
+// ---- footprints (record + payload bytes) that run the register-resident kernel ---------------
+// A single-GPU, ticket-ranked pass of footprint (ES, PL) runs this kernel with the tile Cfg2<ES, PL>
+// where PreferV2<ES, PL> holds, and scatter_kernel otherwise: flipped per footprint by measurement
+// (profiles/r2_variants.md).  Every other footprint measured slower than the staging kernel
+// (tools/footprints.py).
 template <int ES, int PL> struct PreferV2 { static constexpr bool value = false; };
 // 8-byte records without a payload lane (u64 / i64 / f64 keys, {u32 key, u32 payload} records):
-// 256 threads x 32 records, two CTAs per SM, count + ticket placement -- 4.01 ms per pass of 1 B u64
-// keys against 4.22 ms for the staging kernel, which has room for only one CTA per SM.
-template <> struct PreferV2<8, 0> { static constexpr bool value = true; };
-// u32 keys + u32 index lane (radix_sort_rank on 32-bit keys): 18.6 vs 19.8 ms per 1 B-key rank sort.
-// Every other footprint measured slower than the staging kernel (tools/footprints.py, profiles/r2_variants.md).
-template <> struct PreferV2<4, 4> { static constexpr bool value = true; };
+// 256 threads x 36 records, two CTAs per SM -- 3.95 ms per pass of 1 B u64 keys (4.01 ms at 32
+// records per thread) against 4.22 ms for the staging kernel, which has room for only one CTA per SM.
+template <> struct PreferV2<8, 0> {
+	static constexpr bool value = true;
+	using Cfg = CfgT<256, 36, 2, 8>;
+};
+// u32 keys + u32 index lane (radix_sort_rank on 32-bit keys), 256 threads x 32 records: 18.6 vs
+// 19.8 ms per 1 B-key rank sort.
+template <> struct PreferV2<4, 4> {
+	static constexpr bool value = true;
+	using Cfg = CfgT<256, 32, 2, 8>;
+};
+template <int ES, int PL> using Cfg2 = typename PreferV2<ES, PL>::Cfg;
 
 // Streaming load: every record is read exactly once per pass.
 template <typename R> __device__ __forceinline__ R ld_stream(const R *p) { return __ldcs(p); }
@@ -130,13 +97,8 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter2_kerne
 	constexpr int TILE = SM::kTile;
 	constexpr int WARPS = SM::kWarps;
 	constexpr int LB = Cfg::kLookback;
-#ifdef RSX_WRITE_BATCH
-	constexpr int kWriteBatch = RSX_WRITE_BATCH;
-#else
-	constexpr int kWriteBatch = 2;
-#endif
+	constexpr int kWriteBatch = 2; // records per write-out batch (see scatter_kernel)
 	constexpr uint32_t FULL = 0xFFFFFFFFu;
-	static_assert(ITEMS * 32 <= 65536, "two ranks are packed into one register");
 	static_assert(THREADS >= kBins && THREADS % 32 == 0, "one digit thread per bin: the digit scan synchronises 256 threads");
 
 	extern __shared__ __align__(128) unsigned char smem[];
@@ -228,9 +190,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter2_kerne
 		}
 		__syncwarp();
 
-		// ---- 1. stable rank inside the warp: items ascending, lanes ascending (ticket) ----
-		constexpr int MODE = Cfg::kMode;
-		uint32_t rk[MODE == 0 ? (ITEMS + 1) / 2 : 1]; // MODE 0: two 16-bit ranks per register
+		// ---- 1. count per warp and digit; the previous tile's hot digit is counted by a vote ----
 		uint32_t hotcnt = 0;
 		const uint32_t hot = s_misc[9];
 		{
@@ -239,15 +199,7 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter2_kerne
 				const uint32_t d = tile_digit<ES, DM>(p, key[i], dd);
 				const bool is_hot = d == hot;
 				const uint32_t m = __ballot_sync(FULL, is_hot);
-				if constexpr (MODE == 0) {
-					const uint32_t r = ticket_unless(&wh[d], is_hot, hotcnt + __popc(m & lt));
-					if (i & 1)
-						rk[i >> 1] |= r << 16;
-					else
-						rk[i >> 1] = r;
-				} else {
-					count_unless(&wh[d], is_hot);
-				}
+				count_unless(&wh[d], is_hot);
 				hotcnt += __popc(m);
 			}
 			if (lane == 0)
@@ -297,31 +249,21 @@ __global__ void __launch_bounds__(Cfg::kThreads, Cfg::kMinBlocks) scatter2_kerne
 		}
 		__syncthreads(); // (C)
 
-		// ---- 3. records / payloads to their tile-sorted slot ----
-		if constexpr (MODE == 0) {
+		// ---- 3. records / payloads to their tile-sorted slot: stable rank inside the warp (items
+		//      ascending, lanes ascending) in the same sweep order as the count, so the ticket
+		//      returns the slot itself ----
+		uint32_t hotpos = wh[hot];
+		__syncwarp();
 #pragma unroll
-			for (int i = 0; i < ITEMS; ++i) {
-				const uint32_t r = (i & 1) ? (rk[i >> 1] >> 16) : (rk[i >> 1] & 0xFFFFu);
-				const uint32_t pos = wh[tile_digit<ES, DM>(p, key[i], dd)] + r;
-				s_rec[pos] = key[i];
-				if constexpr (PL != 0)
-					s_pl[pos] = synth ? (P)(base + t0 + i * 32) : pay[i];
-			}
-		} else {
-			// same sweep order as the count: the ticket now returns the slot itself
-			uint32_t hotpos = wh[hot];
-			__syncwarp();
-#pragma unroll
-			for (int i = 0; i < ITEMS; ++i) {
-				const uint32_t d = tile_digit<ES, DM>(p, key[i], dd);
-				const bool is_hot = d == hot;
-				const uint32_t m = __ballot_sync(FULL, is_hot);
-				const uint32_t pos = ticket_unless(&wh[d], is_hot, hotpos + __popc(m & lt));
-				hotpos += __popc(m);
-				s_rec[pos] = key[i];
-				if constexpr (PL != 0)
-					s_pl[pos] = synth ? (P)(base + t0 + i * 32) : pay[i];
-			}
+		for (int i = 0; i < ITEMS; ++i) {
+			const uint32_t d = tile_digit<ES, DM>(p, key[i], dd);
+			const bool is_hot = d == hot;
+			const uint32_t m = __ballot_sync(FULL, is_hot);
+			const uint32_t pos = ticket_unless(&wh[d], is_hot, hotpos + __popc(m & lt));
+			hotpos += __popc(m);
+			s_rec[pos] = key[i];
+			if constexpr (PL != 0)
+				s_pl[pos] = synth ? (P)(base + t0 + i * 32) : pay[i];
 		}
 
 		// ---- 4. decoupled look-back, one chain per digit; the first round is split over two

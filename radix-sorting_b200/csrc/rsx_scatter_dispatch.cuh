@@ -1,5 +1,5 @@
 // rsx_scatter_dispatch.cuh -- picks the scatter kernel for one pass: record size, payload lane,
-// float digits, 32/64-bit offsets, rank mode, fused partition+exchange, tuning variant.
+// float digits, 32/64-bit offsets, rank mode, fused partition+exchange.
 #pragma once
 
 #include "rsx_scatter.cuh"
@@ -7,89 +7,26 @@
 
 namespace rsx {
 
-// scatter_variant values: 0 default, 1..kNumVariants-1 staging-kernel geometries (plain 4/8-byte
-// keys), 10 + V register-resident kernel geometry V.
-constexpr int kVariant2Base = 10;
-inline bool variant_is_v2(int v) { return v >= kVariant2Base && v < kVariant2Base + kNumVariants2; }
-
-template <int ES, int PL, int DM, typename OffT>
-cudaError_t launch_scatter2_v(const ScatterParams &sp, int num_sms, cudaStream_t st, int v2) {
-	if constexpr ((ES == 4 || ES == 8) && PL == 0 && DM == DIGIT_PLAIN && sizeof(OffT) == 4) {
-		switch (v2) {
-		case 1: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 1>>(sp, num_sms, st);
-		case 2: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 2>>(sp, num_sms, st);
-		case 3: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 3>>(sp, num_sms, st);
-		case 4: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 4>>(sp, num_sms, st);
-		case 5: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 5>>(sp, num_sms, st);
-		case 6: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 6>>(sp, num_sms, st);
-		case 7: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 7>>(sp, num_sms, st);
-		case 8: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 8>>(sp, num_sms, st);
-		case 9: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 9>>(sp, num_sms, st);
-		case 10: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 10>>(sp, num_sms, st);
-		case 11: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 11>>(sp, num_sms, st);
-		case 12: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 12>>(sp, num_sms, st);
-		case 13: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 13>>(sp, num_sms, st);
-		case 14: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 14>>(sp, num_sms, st);
-		case 15: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 15>>(sp, num_sms, st);
-		case 16: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 16>>(sp, num_sms, st);
-		case 17: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 17>>(sp, num_sms, st);
-		case 18: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 18>>(sp, num_sms, st);
-		case 19: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 19>>(sp, num_sms, st);
-		case 20: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 20>>(sp, num_sms, st);
-		case 21: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 21>>(sp, num_sms, st);
-		case 22: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 22>>(sp, num_sms, st);
-		case 23: return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 23>>(sp, num_sms, st);
-		default: break;
-		}
-	}
-	return launch_scatter2_c<ES, PL, DM, OffT, Cfg2V<ES, PL, 0>>(sp, num_sms, st);
-}
-
-// true: the register-resident kernel runs this (single-GPU, ticket-ranked) pass
-template <int ES, int PL> inline bool pass_uses_v2(int variant) {
-	return variant_is_v2(variant) || (variant == 0 && PreferV2<ES, PL>::value);
-}
-
-template <int ES, int PL, int DM, bool FUSED, typename OffT, int RANK>
-cudaError_t launch_scatter_r(const ScatterParams &sp, int num_sms, cudaStream_t st) {
-	if constexpr ((ES == 4 || ES == 8) && PL == 0 && DM == DIGIT_PLAIN && !FUSED && RANK == RANK_TICKET && sizeof(OffT) == 4) {
-		switch (scatter_variant()) {
-		case 1: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 1>>(sp, num_sms, st);
-		case 2: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 2>>(sp, num_sms, st);
-		case 3: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 3>>(sp, num_sms, st);
-		case 4: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 4>>(sp, num_sms, st);
-		case 5: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 5>>(sp, num_sms, st);
-		case 6: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 6>>(sp, num_sms, st);
-		case 7: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 7>>(sp, num_sms, st);
-		case 8: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 8>>(sp, num_sms, st);
-		case 9: return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfgV<ES, PL, 9>>(sp, num_sms, st);
-		default: break;
-		}
-	}
-	if constexpr (FUSED)
-		return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, FusedCfg<ES, PL>>(sp, num_sms, st);
-	else
-		return launch_scatter_c<ES, PL, DM, FUSED, OffT, RANK, ScatterCfg<ES, PL>>(sp, num_sms, st);
-}
-
 template <int ES, int PL, int DM, typename OffT>
 cudaError_t launch_scatter_t(const ScatterParams &sp, int num_sms, cudaStream_t st) {
 	const bool ticket = rank_mode() == RANK_TICKET;
 	if (sp.dest_base != nullptr) { // fused partition + exchange (records only)
 		if constexpr (PL == 0)
-			return ticket ? launch_scatter_r<ES, PL, DM, true, OffT, RANK_TICKET>(sp, num_sms, st)
-			              : launch_scatter_r<ES, PL, DM, true, OffT, RANK_BALLOT>(sp, num_sms, st);
+			return ticket ? launch_scatter_c<ES, PL, DM, true, OffT, RANK_TICKET, FusedCfg<ES, PL>>(sp, num_sms, st)
+			              : launch_scatter_c<ES, PL, DM, true, OffT, RANK_BALLOT, FusedCfg<ES, PL>>(sp, num_sms, st);
 		else
 			return cudaErrorInvalidValue;
 	}
 	if constexpr (DM == DIGIT_SPLIT) {
 		return cudaErrorInvalidValue; // key-range routing exists in fused form only
 	} else {
-		const int v = scatter_variant();
-		if (ticket && pass_uses_v2<ES, PL>(v))
-			return launch_scatter2_v<ES, PL, DM, OffT>(sp, num_sms, st, variant_is_v2(v) ? v - kVariant2Base : 0);
-		return ticket ? launch_scatter_r<ES, PL, DM, false, OffT, RANK_TICKET>(sp, num_sms, st)
-		              : launch_scatter_r<ES, PL, DM, false, OffT, RANK_BALLOT>(sp, num_sms, st);
+		if (ticket) { // the register-resident kernel ranks by ticket only
+			if constexpr (PreferV2<ES, PL>::value)
+				return launch_scatter2_c<ES, PL, DM, OffT, Cfg2<ES, PL>>(sp, num_sms, st);
+			else
+				return launch_scatter_c<ES, PL, DM, false, OffT, RANK_TICKET, ScatterCfg<ES, PL>>(sp, num_sms, st);
+		}
+		return launch_scatter_c<ES, PL, DM, false, OffT, RANK_BALLOT, ScatterCfg<ES, PL>>(sp, num_sms, st);
 	}
 }
 
@@ -123,6 +60,5 @@ cudaError_t launch_scatter_es(const ScatterParams &sp, int payload_bytes, bool i
 	}
 	return cudaErrorInvalidValue;
 }
-
 
 } // namespace rsx

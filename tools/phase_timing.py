@@ -10,13 +10,11 @@ import types
 mod = importlib.import_module("radix-sorting_b200")
 dbg = C.CDLL(os.path.join(ROOT, "tools", "dbg", "librsx_dbg.so"))
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 1_000_000_000
-variant = int(sys.argv[2]) if len(sys.argv) > 2 else 0
-kb = int(sys.argv[3]) if len(sys.argv) > 3 else 4
+kb = int(sys.argv[2]) if len(sys.argv) > 2 else 4
 dt = torch.int32 if kb == 4 else torch.int64
 src = torch.empty(n, dtype=dt, device="cuda"); aux = torch.empty_like(src); pristine = torch.empty_like(src)
 mod.fill_keys(pristine, seed=2)
 L = mod.RsxLayout(kb, 0, kb, 0, 0)
-dbg.rsx_set_option(b"scatter_variant", variant)
 res = C.c_void_p(); rep = mod.RsxReport()
 names = ["load/wait stage", "rank (atoms)", "barrier A", "digit phase", "barrier C", "scatter->smem", "look-back", "barrier D", "write-out", "loop top", "lb rounds", "lb polls", "CTAs"]
 for it in range(3):
@@ -29,7 +27,7 @@ for it in range(3):
 tiles_total = None
 ctas = out[12]
 tot = sum(out[k] for k in range(10))
-print(f"n={n} kb={kb} variant={variant} CTAs(sum over {rep.ncols} passes)={ctas}")
+print(f"n={n} kb={kb} CTAs(sum over {rep.ncols} passes)={ctas}")
 for k in range(10):
     print(f"  {names[k]:18s} {out[k]/ctas:12.0f} cyc/CTA  {100*out[k]/tot:5.1f}%")
 print(f"  lb rounds {out[10]}  polls {out[11]}")
