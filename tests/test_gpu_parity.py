@@ -34,7 +34,8 @@ def to_dev(torch, a: np.ndarray):
 
 
 def kf_for(rsx, tname, descending=False):
-    t = TYPES[tname]
+    """KeyFunc of TYPES[tname], or of `tname` itself when it is a pyoracle.ElemType."""
+    t = TYPES[tname] if isinstance(tname, str) else tname
     return rsx.KeyFunc(t.kdf_kind, descending, t.record_bytes, t.key_offset, t.key_bytes)
 
 
