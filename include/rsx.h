@@ -120,6 +120,29 @@ int rsx_sort_segments(void *src, void *aux, size_t n, const uint64_t *offsets, s
 int rsx_sort_rank_segments(const void *src, void *index_buffer, size_t n, const uint64_t *offsets, size_t nseg,
                            const rsx_layout *layout, int idx_bytes, void **result, rsx_report *report, void *stream);
 
+/* ---- top-k: the front of the stable sort without sorting the whole array -----------------------
+ * No reference equivalent; what torch.topk(sorted=True) and threshold queries offer.
+ *   content  out[0..k) is byte for byte radix_sort(src)[0..k): ascending by derived key, ties in input
+ *            order.  RSX_FLAG_INVERT gives the k largest, ties still in input order.  Every KDF.
+ *            index_out[0..k) is the first k entries of rsx_sort_rank's stable argsort, written at
+ *            idx_bytes (1, 2, 4 or 8) each.
+ *   buffers  src is never written; out holds k records, index_out k indices.  Nothing else is asked of
+ *            the caller: the scratch is library workspace.
+ *   checks   before any device work: k > n, a bad layout, a record size other than 1/2/4/8/16, idx_bytes
+ *            not in {1, 2, 4, 8}, a NULL out / index_out with k > 0, or out / index_out overlapping src
+ *            -> RSX_ERR_INVALID; n - 1 not fitting idx_bytes -> RSX_ERR_IDX_RANGE; k == 0 -> RSX_OK
+ *            without touching the device.  src and out must be device (or managed) memory
+ *            (RSX_ERR_MIXED_MEMORY otherwise).
+ *   report   kernel_launches: every kernel the call launched (the first call on a device that ranks
+ *            also counts the one-time ranking probe, as rsx_sort does); ncols: the key columns the threshold
+ *            search histogrammed (<= key_bytes; it stops once the bucket it narrows holds exactly the
+ *            records still needed).  Every other field is 0.
+ * Synchronous like rsx_sort.  Cost: up to key_bytes + 1 read-only passes over src plus a sort of k
+ * records; at most 2 * key_bytes + 6 kernel launches (DESIGN.md "Top-k"). */
+int rsx_topk(const void *src, size_t n, size_t k, const rsx_layout *layout, void *out, rsx_report *report, void *stream);
+int rsx_topk_rank(const void *src, size_t n, size_t k, const rsx_layout *layout, int idx_bytes, void *index_out,
+                  rsx_report *report, void *stream);
+
 /* ---- the two halves of the path, exposed for parity tests and profiling --------------------
  * rsx_histogram = phase 1-3 of rs_sort_main (radix_sort.hpp:46-80): one read of the keys
  * producing all key_bytes x 256 digit counts (column-major, BEFORE the exclusive scan, bins

@@ -9,6 +9,7 @@ torch tensors (torch is used for device memory and streams only):
     radix_sort(src, aux, n=None, kf=None)            -> radix_sort.hpp:98-115
     radix_sort_rank(src, index_buffer, n=None, kf=None) -> radix_sort_rank.hpp:97-112
     radix_sort_segments / radix_sort_rank_segments        -> many independent arrays in one call
+    radix_topk / radix_topk_rank                          -> the first k records / indices of the sort
 
 Both return the tensor / half that holds the result, like the reference returns a pointer.
 There is NO CPU fallback: importing this module without a built ``librsx.so`` raises, and
@@ -36,7 +37,7 @@ RSX_ERR_WORKSPACE, RSX_ERR_IDX_RANGE, RSX_ERR_MIXED_MEMORY = -4, -5, -6
 
 #: every symbol include/rsx.h declares (tests check that the library exports all of them)
 EXPORTS = [
-    "rsx_sort", "rsx_sort_rank", "rsx_sort_segments", "rsx_sort_rank_segments", "rsx_histogram", "rsx_histogram_column", "rsx_scatter_pass", "rsx_scatter_pass_to",
+    "rsx_sort", "rsx_sort_rank", "rsx_sort_segments", "rsx_sort_rank_segments", "rsx_topk", "rsx_topk_rank", "rsx_histogram", "rsx_histogram_column", "rsx_scatter_pass", "rsx_scatter_pass_to",
     "rsx_split_counts", "rsx_split_pass_to", "rsx_scatter_pass_append", "rsx_histogram_column_sampled", "rsx_sample_keys", "rsx_plan_compaction",
     "rsx_multi_route", "rsx_multi_splitters", "rsx_sort_shard", "rsx_sort_multi",
     "rsx_workspace_bytes",
@@ -138,6 +139,10 @@ def _lib() -> C.CDLL:
     L.rsx_sort_segments.argtypes = [vp, vp, sz, u64p, sz, LP, C.POINTER(vp), RP, vp]
     L.rsx_sort_rank_segments.restype = C.c_int
     L.rsx_sort_rank_segments.argtypes = [vp, vp, sz, u64p, sz, LP, C.c_int, C.POINTER(vp), RP, vp]
+    L.rsx_topk.restype = C.c_int
+    L.rsx_topk.argtypes = [vp, sz, sz, LP, vp, RP, vp]
+    L.rsx_topk_rank.restype = C.c_int
+    L.rsx_topk_rank.argtypes = [vp, sz, sz, LP, C.c_int, vp, RP, vp]
     L.rsx_histogram.restype = C.c_int
     L.rsx_histogram.argtypes = [vp, sz, LP, u64p, u64p, RP, vp]
     L.rsx_histogram_column.restype = C.c_int
@@ -380,6 +385,48 @@ def radix_sort_rank_segments(src, index_buffer, offsets, kf: Optional[KeyFunc] =
         raise RsxError(st, "rsx_sort_rank_segments")
     off_el = (res.value - index_buffer.data_ptr()) // ib_bytes if n else 0
     return index_buffer.view(-1)[off_el:off_el + n]
+
+
+def radix_topk(src, k: int, out, kf: Optional[KeyFunc] = None, *, report: Optional[RsxReport] = None):
+    """The first k records of radix_sort(src), ties in input order (rsx_topk); a descending KeyFunc
+    gives the k largest.  `src`/`out`: device tensors, `out` holds at least k records.  Returns the
+    view of `out` that holds them.  `src` is not modified."""
+    torch = _torch()
+    _check(src, "src"), _check(out, "out")
+    if src.device != out.device:
+        raise ValueError("src and out must be on the same device")
+    kf = kf or default_kdf(src.dtype)
+    L = kf.layout(src.element_size())
+    n = src.numel() * src.element_size() // L.record_bytes
+    if out.numel() * out.element_size() < k * L.record_bytes:
+        raise ValueError("out must hold k records")
+    rep = report if report is not None else RsxReport()
+    with torch.cuda.device(src.device if src.is_cuda else None):
+        st = _lib().rsx_topk(src.data_ptr(), n, k, C.byref(L), out.data_ptr(), C.byref(rep), _stream_ptr(src))
+    if st != RSX_OK:
+        raise RsxError(st, "rsx_topk")
+    return out.view(-1)[:k * L.record_bytes // out.element_size()]
+
+
+def radix_topk_rank(src, k: int, index_out, kf: Optional[KeyFunc] = None, *, report: Optional[RsxReport] = None):
+    """The first k indices of radix_sort_rank(src) (rsx_topk_rank), at index_out's element size
+    (1, 2, 4 or 8 bytes).  Returns index_out's first k entries.  `src` is not modified."""
+    torch = _torch()
+    _check(src, "src"), _check(index_out, "index_out")
+    if src.device != index_out.device:
+        raise ValueError("src and index_out must be on the same device")
+    kf = kf or default_kdf(src.dtype)
+    L = kf.layout(src.element_size())
+    n = src.numel() * src.element_size() // L.record_bytes
+    if index_out.numel() < k:
+        raise ValueError("index_out must hold k entries")
+    rep = report if report is not None else RsxReport()
+    with torch.cuda.device(src.device if src.is_cuda else None):
+        st = _lib().rsx_topk_rank(src.data_ptr(), n, k, C.byref(L), index_out.element_size(), index_out.data_ptr(),
+                                  C.byref(rep), _stream_ptr(src))
+    if st != RSX_OK:
+        raise RsxError(st, "rsx_topk_rank")
+    return index_out.view(-1)[:k]
 
 
 def histogram(src, kf: Optional[KeyFunc] = None):

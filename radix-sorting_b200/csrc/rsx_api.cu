@@ -1344,6 +1344,109 @@ int rsx_sort_rank_segments(const void *src, void *index_buffer, size_t n, const 
 	return sort_segments_common(src, nullptr, index_buffer, idx_bytes, n, offsets, nseg, layout, result, report, stream);
 }
 
+// ---- top-k --------------------------------------------------------------------------------------
+// Threshold search (key_bytes histogram launches, most of them returning at once for random keys),
+// one stable select of the k records in front of the threshold, then the ordinary sort of those k
+// records (rsx_topk.cu).  The search state, the per-chunk counts and the buffers around the sort of k
+// records live in the stage lease; the sort itself uses the workspace lease.
+static int topk_common(const void *src, size_t n, size_t k, const rsx_layout *layout, int idx_bytes, void *out,
+                       rsx_report *rep, void *stream) {
+	const bool ranksort = idx_bytes != 0;
+	KeyDesc kd;
+	int r = check_layout(layout, &kd); // records the tile kernels move directly: 1, 2, 4, 8 or 16 bytes
+	if (r)
+		return r;
+	if (ranksort && !(idx_bytes == 1 || idx_bytes == 2 || idx_bytes == 4 || idx_bytes == 8))
+		return RSX_ERR_INVALID;
+	if (k > n || (k > 0 && (!src || !out)))
+		return RSX_ERR_INVALID;
+	const uint32_t rb = layout->record_bytes;
+	if (k > 0) { // src is never written: the output must not overlap it
+		const unsigned char *a = static_cast<const unsigned char *>(src), *b = static_cast<const unsigned char *>(out);
+		const size_t ob = k * (ranksort ? (size_t)idx_bytes : rb);
+		if (a < b + ob && b < a + n * rb)
+			return RSX_ERR_INVALID;
+	}
+	if (ranksort && !idx_fits(idx_bytes, n))
+		return RSX_ERR_IDX_RANGE;
+	if (rep)
+		memset(rep, 0, sizeof(*rep));
+	if (k == 0)
+		return RSX_OK;
+	int dev;
+	if ((r = current_device(&dev)))
+		return r;
+	PtrKind ks, ko;
+	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(out, &ko)))
+		return r;
+	if (ks != PK_DEVICE || ko != PK_DEVICE)
+		return RSX_ERR_MIXED_MEMORY;
+	cudaStream_t st = static_cast<cudaStream_t>(stream);
+	const unsigned long long l0 = g_launches.load();
+	const int sms = g_dev[dev].num_sms;
+	const TopkChunks g = topk_chunks(src, n, rb, sms);
+	// positions of the selected records (rank form) and the ranks of their sort
+	const int sel_ib = n - 1 <= 0xFFFFFFFFull ? 4 : 8, rank_ib = k - 1 <= 0xFFFFFFFFull ? 4 : 8;
+	// stage: [state | chunk histograms | chunk lt | chunk eq | records | positions | 2k ranks]
+	const size_t off_hist = align_up(sizeof(TopkState), 256);
+	const size_t off_lt = off_hist + align_up((size_t)g.nchunks * kBins * sizeof(uint32_t), 256);
+	const size_t off_eq = off_lt + align_up((size_t)g.nchunks * sizeof(unsigned long long), 256);
+	const size_t off_rec = off_eq + align_up((size_t)g.nchunks * sizeof(unsigned long long), 256);
+	const size_t off_pos = off_rec + align_up(k * rb, 256);
+	const size_t off_ib = off_pos + (ranksort ? align_up(k * (size_t)sel_ib, 256) : 0);
+	const size_t total = off_ib + (ranksort ? 2 * k * (size_t)rank_ib : 0);
+	unsigned char *hbuf = nullptr;
+	if ((r = segment_host_buffer(sizeof(uint32_t), &hbuf)))
+		return r;
+	StageLease SL;
+	if ((r = acquire_stage(SL, dev, total)))
+		return r;
+	SL.inflight = st;
+	SL.has_inflight = true; // drained below on success, by ~StageLease on any failure
+	unsigned char *sp = static_cast<unsigned char *>(SL.ptr);
+	TopkState *s = reinterpret_cast<TopkState *>(sp);
+	auto *clt = reinterpret_cast<unsigned long long *>(sp + off_lt), *ceq = reinterpret_cast<unsigned long long *>(sp + off_eq);
+	CU(cudaMemsetAsync(sp, 0, off_rec, st));
+	for (int c = (int)kd.key_bytes - 1; c >= 0; --c)
+		CU(launch_topk_hist(src, n, k, rb, kd, c, g, s, reinterpret_cast<uint32_t *>(sp + off_hist), clt, ceq, st));
+	// value form: the selection goes straight to `out` and is sorted there, the stage buffer is aux
+	void *sel = ranksort ? static_cast<void *>(sp + off_rec) : out;
+	CU(launch_topk_select(src, n, k, rb, kd, g, s, clt, ceq, sel, ranksort ? sp + off_pos : nullptr, ranksort ? sel_ib : 0, st));
+	CU(cudaMemcpyAsync(hbuf, &s->ncols, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+	void *res = nullptr;
+	rsx_report srep;
+	if (!ranksort) {
+		if (k >= 2) {
+			if ((r = sort_device(out, sp + off_rec, k, layout, kd, &res, &srep, st, dev, false)))
+				return r;
+			if (res != out)
+				CU(cudaMemcpyAsync(out, res, k * rb, cudaMemcpyDeviceToDevice, st));
+		}
+	} else {
+		if (k >= 2 && (r = rank_device(sel, sp + off_ib, k, layout, kd, rank_ib, &res, &srep, st, dev, false)))
+			return r;
+		CU(launch_topk_gather(res, rank_ib, sp + off_pos, sel_ib, out, idx_bytes, k, sms, st));
+	}
+	CU(cudaStreamSynchronize(st));
+	SL.has_inflight = false;
+	if (rep) {
+		rep->ncols = *reinterpret_cast<const uint32_t *>(hbuf);
+		rep->kernel_launches = (uint32_t)(g_launches.load() - l0);
+	}
+	return RSX_OK;
+}
+
+int rsx_topk(const void *src, size_t n, size_t k, const rsx_layout *layout, void *out, rsx_report *report, void *stream) {
+	return topk_common(src, n, k, layout, 0, out, report, stream);
+}
+
+int rsx_topk_rank(const void *src, size_t n, size_t k, const rsx_layout *layout, int idx_bytes, void *index_out,
+                  rsx_report *report, void *stream) {
+	if (idx_bytes == 0)
+		return RSX_ERR_INVALID;
+	return topk_common(src, n, k, layout, idx_bytes, index_out, report, stream);
+}
+
 // ---- halves of the path, for parity tests and profiling ------------------------------------------
 int rsx_histogram(const void *src, size_t n, const rsx_layout *layout, uint64_t *hist_out,
                   uint64_t *descents_out, rsx_report *rep, void *stream) {

@@ -142,6 +142,41 @@ cudaError_t launch_segment_groups(const void *src, void *out_even, void *out_odd
                                   uint32_t record_bytes, const KeyDesc &kd, const SegGroup *groups, size_t ngroups,
                                   const uint32_t *segtab, const Ctl *ctl, cudaStream_t st);
 
+// top-k (rsx_topk.cu).  The threshold search is MSD radix select on the derived key: one histogram
+// launch per column, from the top column down, over the records whose derived-key bits above the
+// column equal `prefix`.  The last CTA of each launch picks the bucket that holds the k-th record and
+// updates this block, so every launch is enqueued without the host waiting.  Zeroed before the search.
+struct TopkState {
+	unsigned long long hist[kBins]; // the current column's counts (reset by the deciding CTA)
+	unsigned long long prefix;      // derived-key bits of columns col .. key_bytes-1 of the k-th record
+	unsigned long long less;        // records whose derived key sorts below that prefix
+	uint32_t ticket;                // CTAs done with the current column (reset by the deciding CTA)
+	uint32_t done;                  // the prefix bucket holds exactly k - less records, or col == 0
+	uint32_t ncols;                 // columns histogrammed
+	uint32_t col;                   // the last column histogrammed
+};
+// Every top-k kernel of one call splits the records the same way: chunk j is a contiguous range, so
+// per-chunk counts of the search passes give each CTA of the select its output offsets.  Records
+// [0, head) go to chunk 0 and the tail that does not fill a 16-byte vector to the last chunk.
+struct TopkChunks {
+	size_t head, n_vec, per; // unaligned head records, 16-byte vectors after them, vectors per chunk
+	uint32_t nchunks;
+};
+TopkChunks topk_chunks(const void *src, size_t n, uint32_t record_bytes, int num_sms);
+// chunk_hist: nchunks x 256 counts of this column; chunk_lt / chunk_eq: per chunk, records below the
+// prefix and records equal to it (zeroed before the search)
+cudaError_t launch_topk_hist(const void *src, size_t n, size_t k, uint32_t record_bytes, const KeyDesc &kd, int col,
+                             const TopkChunks &g, TopkState *s, uint32_t *chunk_hist, unsigned long long *chunk_lt,
+                             unsigned long long *chunk_eq, cudaStream_t st);
+// out[0, less): records below the prefix in input order; out[less, k): the first k - less records
+// equal to it.  sel_idx_bytes 4 or 8: each record's input position goes to sel_idx; 0: none.
+cudaError_t launch_topk_select(const void *src, size_t n, size_t k, uint32_t record_bytes, const KeyDesc &kd, const TopkChunks &g,
+                               const TopkState *s, const unsigned long long *chunk_lt, const unsigned long long *chunk_eq,
+                               void *out, void *sel_idx, int sel_idx_bytes, cudaStream_t st);
+// index_out[i] = sel_idx[rank[i]] (rank == nullptr: sel_idx[i]), narrowed to idx_bytes
+cudaError_t launch_topk_gather(const void *rank, int rank_bytes, const void *sel_idx, int sel_idx_bytes, void *index_out,
+                               int idx_bytes, size_t k, int num_sms, cudaStream_t st);
+
 // rank-sort helpers
 cudaError_t launch_iota_if_early(void *index_buffer, int idx_bytes, size_t n, const Ctl *ctl,
                                  cudaStream_t st);
