@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <vector>
 
@@ -82,18 +83,23 @@ int fail_cuda(cudaError_t e, const char *what) {
 			return fail_cuda(e_, #call);          \
 	} while (0)
 
-// ---- per-device state: SM count, grow-only workspace, pinned read-back slot -------------------
+// ---- per-device state: SM count, grow-only workspace and staging buffers ----------------------
+// A cached grow-only device buffer, used by one call at a time (guarded by `busy`).
+struct Slot {
+	void *ptr = nullptr;
+	size_t bytes = 0;
+	bool busy = false;
+	Ctl *pinned = nullptr; // workspace slot only: the mapped pinned pass table + read-back area
+};
+enum SlotId { WORKSPACE, STAGE };
 struct DeviceState {
 	std::mutex mu;
 	int num_sms = 0;
 	int rank_mode = -1; // -1 = not probed yet
-	void *ws = nullptr;
-	size_t ws_bytes = 0;
-	bool busy = false;
-	Ctl *pinned = nullptr; // one slot per device is enough: guarded by `busy`
-	void *stage = nullptr; // device staging for host-pointer calls (grow-only, like ws)
-	size_t stage_bytes = 0;
-	bool stage_busy = false;
+	// WORKSPACE: look-back state, head and rank-sort buffers.  STAGE: device copies of host buffers
+	// (cached so that a caller sorting host arrays repeatedly does not pay cudaMalloc/cudaFree of
+	// gigabytes on every call) and the scratch of segmented sorts and top-k around their inner sorts.
+	Slot slot[2];
 };
 constexpr int kMaxDevices = 64;
 DeviceState g_dev[kMaxDevices];
@@ -135,16 +141,16 @@ int probe_rank_mode(int dev) {
 // copies into pageable memory are staged by the driver and cost tens of microseconds more).
 constexpr size_t kPinnedReadback = 256, kPinnedBytes = kPinnedReadback + sizeof(unsigned long long) * kMaxCols * kBins;
 
+// One call's use of a slot: the cached buffer, or a private one when another host thread holds it.
 struct Lease {
 	int dev = -1;
+	Slot *cached = nullptr; // null: ptr (and pinned, for a workspace) are this call's own
 	void *ptr = nullptr;
 	Ctl *pinned = nullptr;
 	unsigned long long *readback() const { return reinterpret_cast<unsigned long long *>(reinterpret_cast<unsigned char *>(pinned) + kPinnedReadback); }
-	bool cached = false;
-	bool own_pinned = false;
-	// Set once kernels that use the leased memory have been enqueued; cleared by the final
-	// synchronising read-back.  If a call fails in between, the destructor drains the stream
-	// before another host thread can be handed the same workspace.
+	// Set once copies or kernels that use the leased memory have been enqueued; cleared once the
+	// stream has been synchronised.  If a call fails in between, the destructor drains the stream
+	// before another host thread can be handed the same buffer.
 	cudaStream_t inflight = nullptr;
 	bool has_inflight = false;
 	void enqueued(cudaStream_t st) { inflight = st; has_inflight = true; }
@@ -158,91 +164,53 @@ struct Lease {
 		}
 		if (cached) {
 			std::lock_guard<std::mutex> lk(g_dev[dev].mu);
-			g_dev[dev].busy = false;
+			cached->busy = false;
 		} else {
 			if (ptr)
 				cudaFree(ptr);
-			if (own_pinned && pinned)
+			if (pinned)
 				cudaFreeHost(pinned);
 		}
 	}
 };
 
-// Device staging buffer for host-pointer calls: cached so that a drop-in caller sorting host
-// arrays repeatedly does not pay cudaMalloc/cudaFree of gigabytes on every call.
-struct StageLease {
-	int dev = -1;
-	void *ptr = nullptr;
-	bool cached = false;
-	cudaStream_t inflight = nullptr;
-	bool has_inflight = false;
-	~StageLease() {
-		if (dev < 0)
-			return;
-		if (has_inflight) { // a failed call may leave copies / kernels running on the staging buffer
-			cudaStreamSynchronize(inflight);
-			(void)cudaGetLastError();
-		}
-		if (cached) {
-			std::lock_guard<std::mutex> lk(g_dev[dev].mu);
-			g_dev[dev].stage_busy = false;
-		} else if (ptr) {
-			cudaFree(ptr);
-		}
-	}
-};
-
-int acquire_stage(StageLease &L, int dev, size_t bytes) {
+int acquire(Lease &L, int dev, SlotId id, size_t bytes) {
 	DeviceState &D = g_dev[dev];
+	Slot &S = D.slot[id];
 	L.dev = dev;
 	std::unique_lock<std::mutex> lk(D.mu);
-	if (!D.stage_busy) {
-		if (D.stage_bytes < bytes) {
-			if (D.stage) {
-				cudaFree(D.stage);
-				D.stage = nullptr;
-				D.stage_bytes = 0;
+	if (!S.busy) {
+		if (S.bytes < bytes) {
+			if (S.ptr) {
+				cudaFree(S.ptr);
+				S.ptr = nullptr;
+				S.bytes = 0;
 			}
-			CU(cudaMalloc(&D.stage, bytes));
-			D.stage_bytes = bytes;
+			CU(cudaMalloc(&S.ptr, bytes));
+			S.bytes = bytes;
 		}
-		D.stage_busy = true;
-		L.ptr = D.stage;
-		L.cached = true;
-		return RSX_OK;
-	}
-	lk.unlock();
-	CU(cudaMalloc(&L.ptr, bytes));
-	return RSX_OK;
-}
-
-int acquire(Lease &L, int dev, size_t bytes) {
-	DeviceState &D = g_dev[dev];
-	L.dev = dev;
-	std::unique_lock<std::mutex> lk(D.mu);
-	if (!D.busy) {
-		if (D.ws_bytes < bytes) {
-			if (D.ws) {
-				cudaFree(D.ws);
-				D.ws = nullptr;
-				D.ws_bytes = 0;
-			}
-			CU(cudaMalloc(&D.ws, bytes));
-			D.ws_bytes = bytes;
-		}
-		if (!D.pinned)
-			CU(cudaHostAlloc((void **)&D.pinned, kPinnedBytes, cudaHostAllocMapped));
-		D.busy = true;
-		L.ptr = D.ws;
-		L.pinned = D.pinned;
-		L.cached = true;
+		if (id == WORKSPACE && !S.pinned)
+			CU(cudaHostAlloc((void **)&S.pinned, kPinnedBytes, cudaHostAllocMapped));
+		S.busy = true;
+		L.ptr = S.ptr;
+		L.pinned = S.pinned;
+		L.cached = &S;
 		return RSX_OK;
 	}
 	lk.unlock(); // another host thread is sorting on this device: private scratch for this call
 	CU(cudaMalloc(&L.ptr, bytes));
-	CU(cudaHostAlloc((void **)&L.pinned, kPinnedBytes, cudaHostAllocMapped));
-	L.own_pinned = true;
+	if (id == WORKSPACE)
+		CU(cudaHostAlloc((void **)&L.pinned, kPinnedBytes, cudaHostAllocMapped));
 	return RSX_OK;
+}
+
+// rsx_release: the buffer of a slot no call is using goes back to the driver.
+void free_if_idle(Slot &S) {
+	if (!S.busy && S.ptr) {
+		cudaFree(S.ptr);
+		S.ptr = nullptr;
+		S.bytes = 0;
+	}
 }
 
 // ---- layout ---------------------------------------------------------------------------------
@@ -319,6 +287,27 @@ int ptr_kind(const void *p, PtrKind *k) {
 	return RSX_OK;
 }
 
+// The buffers a and b (b may be null) must all be device memory; with `common`, they may instead
+// all be host memory, and *common receives their kind.
+int check_residency(PtrKind *common, const void *a, const void *b = nullptr) {
+	PtrKind ka, kb = PK_DEVICE;
+	int r;
+	if ((r = ptr_kind(a, &ka)) || (b && (r = ptr_kind(b, &kb))))
+		return r;
+	if (common ? ka != kb : (ka != PK_DEVICE || kb != PK_DEVICE))
+		return RSX_ERR_MIXED_MEMORY;
+	if (common)
+		*common = ka;
+	return RSX_OK;
+}
+
+bool overlaps(const void *a, size_t abytes, const void *b, size_t bbytes) {
+	const unsigned char *pa = static_cast<const unsigned char *>(a), *pb = static_cast<const unsigned char *>(b);
+	return pa < pb + bbytes && pb < pa + abytes;
+}
+
+bool valid_idx_bytes(int b) { return b == 1 || b == 2 || b == 4 || b == 8; }
+
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 struct Plan {
@@ -334,9 +323,10 @@ struct Plan {
 	int n_rec_bufs;
 };
 
-void make_plan(Plan &P, size_t n, const rsx_layout *L, const KeyDesc &kd, int rank_idx_bytes, int forced_pl = -1) {
+Plan make_plan(size_t n, uint32_t record_bytes, const KeyDesc &kd, int rank_idx_bytes, int forced_pl = -1) {
+	Plan P;
 	P.kd = kd;
-	P.rb = L->record_bytes;
+	P.rb = record_bytes;
 	P.n = n;
 	P.pl_bytes = forced_pl >= 0 ? forced_pl : rank_idx_bytes == 0 ? 0 : (rank_idx_bytes == 8 ? 8 : 4);
 	P.geo = scatter_geometry(P.rb, P.pl_bytes);
@@ -367,14 +357,17 @@ void make_plan(Plan &P, size_t n, const rsx_layout *L, const KeyDesc &kd, int ra
 		}
 	}
 	P.total = off;
+	return P;
 }
 
-int run_scatter(const PassBuffers &pb, const Plan &P, int col, unsigned char *wsp, bool forced, bool single,
-                int num_sms, cudaStream_t st) {
+// The workspace of a call that runs no pass: the head, behind one tile's look-back rows per column.
+Plan head_plan(uint32_t record_bytes, const KeyDesc &kd) { return make_plan(2, record_bytes, kd, 0); }
+
+int run_scatter(const PassBuffers &pb, const Plan &P, int col, unsigned char *wsp, bool forced, int num_sms,
+                cudaStream_t st, const Exchange &ex = {}) {
 	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	(void)single;
 	CU(launch_scatter(pb, P.n, P.rb, P.pl_bytes, P.kd, col, ws, forced, wsp + (size_t)col * P.status_bytes,
-	                  &ws->tickets[col], P.wide, num_sms, st));
+	                  &ws->tickets[col], P.wide, num_sms, st, ex));
 	return RSX_OK;
 }
 
@@ -397,7 +390,7 @@ int enqueue_front(const void *src, const Plan &P, unsigned char *wsp, Ctl *host_
 
 int enqueue_passes(const PassBuffers &pb, const Plan &P, unsigned char *wsp, int num_sms, cudaStream_t st) {
 	for (uint32_t c = 0; c < P.kd.key_bytes; ++c) {
-		int r = run_scatter(pb, P, (int)c, wsp, false, false, num_sms, st);
+		int r = run_scatter(pb, P, (int)c, wsp, false, num_sms, st);
 		if (r)
 			return r;
 		prof_mark(st);
@@ -408,20 +401,23 @@ int enqueue_passes(const PassBuffers &pb, const Plan &P, unsigned char *wsp, int
 // The pass table (which buffer holds the result, radix_sort.hpp:89-92) reaches the host without a
 // copy: the setup kernel (or the single-CTA kernel) also stores it into the lease's mapped pinned
 // slot, so the host only has to wait for the stream.
-int read_ctl(Lease &L, cudaStream_t st, unsigned long long launches0, rsx_report *rep, bool staged) {
-	Ctl *pinned = L.pinned;
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	prof_collect();
+void fill_report(rsx_report *rep, const Ctl &c, unsigned long long launches0, bool staged) {
 	if (rep) {
-		rep->early_exit = pinned->early_exit;
-		rep->ncols = pinned->early_exit ? 0 : pinned->ncols;
-		rep->live_mask = pinned->early_exit ? 0 : pinned->live_mask;
-		rep->result_in_aux = pinned->early_exit ? 0 : (pinned->ncols & 1u);
+		rep->early_exit = c.early_exit;
+		rep->ncols = c.early_exit ? 0 : c.ncols;
+		rep->live_mask = c.early_exit ? 0 : c.live_mask;
+		rep->result_in_aux = c.early_exit ? 0 : (c.ncols & 1u); // radix_sort.hpp:89-92
 		rep->kernel_launches = (uint32_t)(g_launches.load() - launches0);
 		rep->staged = staged;
 		rep->compacted_passes = 0;
 	}
+}
+
+int read_ctl(Lease &L, cudaStream_t st, unsigned long long launches0, rsx_report *rep, bool staged) {
+	CU(cudaStreamSynchronize(st));
+	L.drained();
+	prof_collect();
+	fill_report(rep, *L.pinned, launches0, staged);
 	return RSX_OK;
 }
 
@@ -431,6 +427,59 @@ void trivial_report(rsx_report *rep) {
 		rep->early_exit = 1;
 	}
 }
+
+// Paths that read their own report back (which buffer holds the result) take a NULL `report` into
+// this one.
+rsx_report *report_or_scratch(rsx_report *rep) {
+	thread_local rsx_report scratch;
+	return rep ? rep : &scratch;
+}
+
+// The prologue of an entry point that runs on the current device: open() looks the device up,
+// lease() takes the workspace for plan P and counts its kernels as in flight from then on.
+struct DeviceCall {
+	int dev = -1, sms = 0;
+	cudaStream_t st = nullptr;
+	Plan P;
+	Lease L;
+	unsigned char *wsp = nullptr;
+	WsHead *ws = nullptr;
+
+	int open(void *stream) {
+		int r = current_device(&dev);
+		if (r)
+			return r;
+		sms = g_dev[dev].num_sms;
+		st = static_cast<cudaStream_t>(stream);
+		return RSX_OK;
+	}
+	int lease(const Plan &plan) {
+		P = plan;
+		int r = acquire(L, dev, WORKSPACE, P.total);
+		if (r)
+			return r;
+		L.enqueued(st);
+		wsp = static_cast<unsigned char *>(L.ptr);
+		ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
+		return RSX_OK;
+	}
+	// Waits for the call's work; the workspace is free for the next call.
+	int finish() {
+		CU(cudaStreamSynchronize(st));
+		L.drained();
+		return RSX_OK;
+	}
+	// Device bytes -> host_out, through the lease's pinned read-back area, after the call's work.
+	int read_back(const void *from, size_t bytes, void *host_out) {
+		L.enqueued(st);
+		CU(cudaMemcpyAsync(L.readback(), from, bytes, cudaMemcpyDeviceToHost, st));
+		int r = finish();
+		if (r)
+			return r;
+		memcpy(host_out, L.readback(), bytes);
+		return RSX_OK;
+	}
+};
 
 } // namespace
 
@@ -486,11 +535,7 @@ PassGeometry scatter_geometry(uint32_t record_bytes, int payload_bytes) {
 
 cudaError_t launch_scatter(const PassBuffers &pb, size_t n, uint32_t record_bytes, int payload_bytes,
                            const KeyDesc &kd, int col, const WsHead *ws, bool forced, void *status,
-                           unsigned int *ticket, bool wide, int num_sms, cudaStream_t st,
-                           const unsigned long long *dest_base, const unsigned char *owner,
-                           const unsigned long long *splitters, int nsplit, int ndest,
-                           const unsigned long long *dest_cursor, const unsigned long long *dest_capacity,
-                           unsigned int *overflow) {
+                           unsigned int *ticket, bool wide, int num_sms, cudaStream_t st, const Exchange &ex) {
 	ScatterParams sp;
 	sp.pb = pb;
 	sp.n = n;
@@ -506,18 +551,18 @@ cudaError_t launch_scatter(const PassBuffers &pb, size_t n, uint32_t record_byte
 	sp.ticket = ticket;
 	sp.pad_rec = pad_record(kd);
 	sp.dbg = nullptr;
-	sp.dest_base = dest_base;
-	sp.owner = owner;
-	sp.ndest = (uint32_t)ndest;
-	sp.dest_cursor = dest_cursor;
-	sp.dest_capacity = dest_capacity;
-	sp.overflow = overflow;
+	sp.dest_base = ex.dest_base;
+	sp.owner = ex.owner;
+	sp.ndest = (uint32_t)ex.ndest;
+	sp.dest_cursor = ex.dest_cursor;
+	sp.dest_capacity = ex.dest_capacity;
+	sp.overflow = ex.overflow;
 	// keys-only records: the order inside a (tile, destination) run is free -> TMA bulk stores
-	sp.unordered_runs = (dest_base != nullptr && record_bytes == kd.key_bytes && record_bytes < 16 && g_fused_bulk.load(std::memory_order_relaxed)) ? 1u : 0u;
+	sp.unordered_runs = (ex.dest_base != nullptr && record_bytes == kd.key_bytes && record_bytes < 16 && g_fused_bulk.load(std::memory_order_relaxed)) ? 1u : 0u;
 	sp.kd = kd;
-	sp.nsplit = (uint32_t)nsplit;
+	sp.nsplit = (uint32_t)ex.nsplit;
 	for (int j = 0; j < kMaxSplit; ++j)
-		sp.split[j] = (splitters && j < nsplit) ? splitters[j] : ~0ULL;
+		sp.split[j] = (ex.splitters && j < ex.nsplit) ? ex.splitters[j] : ~0ULL;
 #ifdef RSX_PHASE_TIMING
 	{
 		static unsigned long long *d_dbg = nullptr;
@@ -628,14 +673,9 @@ size_t rsx_workspace_bytes(size_t n, const rsx_layout *layout, int rank_idx_byte
 	bool generic = false;
 	if (check_layout_any(layout, &kd, &generic) != RSX_OK)
 		return 0;
-	Plan P;
-	if (generic) { // the keys are ranked, the records gathered: the passes see key_bytes-sized records
-		const rsx_layout key_layout = {layout->key_bytes, 0, layout->key_bytes, layout->kdf_kind, layout->flags};
-		make_plan(P, n < 2 ? 2 : n, &key_layout, kd, rank_idx_bytes ? rank_idx_bytes : (n <= 0xFFFFFFFFull ? 4 : 8));
-		return P.total;
-	}
-	make_plan(P, n < 2 ? 2 : n, layout, kd, rank_idx_bytes);
-	return P.total;
+	if (generic) // the keys are ranked, the records gathered: the passes see key_bytes-sized records
+		return make_plan(n < 2 ? 2 : n, layout->key_bytes, kd, rank_idx_bytes ? rank_idx_bytes : (n <= 0xFFFFFFFFull ? 4 : 8)).total;
+	return make_plan(n < 2 ? 2 : n, layout->record_bytes, kd, rank_idx_bytes).total;
 }
 
 int rsx_reserve(size_t bytes) {
@@ -644,7 +684,7 @@ int rsx_reserve(size_t bytes) {
 	if (r)
 		return r;
 	Lease L;
-	return acquire(L, dev, bytes);
+	return acquire(L, dev, WORKSPACE, bytes);
 }
 
 void rsx_release(void) {
@@ -653,16 +693,8 @@ void rsx_release(void) {
 		return;
 	DeviceState &D = g_dev[dev];
 	std::lock_guard<std::mutex> lk(D.mu);
-	if (!D.busy && D.ws) {
-		cudaFree(D.ws);
-		D.ws = nullptr;
-		D.ws_bytes = 0;
-	}
-	if (!D.stage_busy && D.stage) {
-		cudaFree(D.stage);
-		D.stage = nullptr;
-		D.stage_bytes = 0;
-	}
+	for (Slot &S : D.slot)
+		free_if_idle(S);
 }
 
 // ---- key compaction (N4) ---------------------------------------------------------------------------
@@ -761,41 +793,44 @@ static int sort_compacted(void *src, void *aux, const Plan &P, unsigned char *ws
 }
 
 // ---- value sort --------------------------------------------------------------------------------
+// Value or rank sort of an input that fits one CTA: one launch (rsx_small.cu), the pass table read
+// back like the multi-kernel path's.
+static bool fits_one_cta(size_t n, uint32_t record_bytes, bool ranksort) {
+	return g_small_path.load(std::memory_order_relaxed) && n <= small_sort_capacity(record_bytes, ranksort);
+}
+static int sort_one_cta(const void *src, void *out_even, void *out_odd, void *ib, int idx_bytes, size_t n, uint32_t record_bytes,
+                        const KeyDesc &kd, rsx_report *rep, cudaStream_t st, int dev, bool staged, unsigned long long launches0) {
+	Lease L;
+	int r = acquire(L, dev, WORKSPACE, sizeof(WsHead) + 256);
+	if (r)
+		return r;
+	L.enqueued(st);
+	prof_mark(st, true);
+	CU(launch_small_sort(src, out_even, out_odd, ib, idx_bytes, n, record_bytes, kd, L.pinned, st));
+	prof_mark(st);
+	return read_ctl(L, st, launches0, rep, staged);
+}
+
+// rep must not be NULL (report_or_scratch).
 static int sort_device(void *src, void *aux, size_t n, const rsx_layout *layout, const KeyDesc &kd,
                        void **result, rsx_report *rep, cudaStream_t st, int dev, bool staged) {
 	const unsigned long long l0 = g_launches.load();
-	if (g_small_path.load(std::memory_order_relaxed) && n <= small_sort_capacity(layout->record_bytes, false)) {
-		// one CTA, one launch (rsx_small.cu)
-		Lease L;
-		int r = acquire(L, dev, sizeof(WsHead) + 256);
-		if (r)
-			return r;
-		L.enqueued(st);
-		prof_mark(st, true);
-		CU(launch_small_sort(src, src, aux, nullptr, 0, n, layout->record_bytes, kd, L.pinned, st));
-		prof_mark(st);
-		rsx_report local;
-		if (!rep)
-			rep = &local;
-		if ((r = read_ctl(L, st, l0, rep, staged)))
+	int r;
+	if (fits_one_cta(n, layout->record_bytes, false)) {
+		if ((r = sort_one_cta(src, src, aux, nullptr, 0, n, layout->record_bytes, kd, rep, st, dev, staged, l0)))
 			return r;
 		*result = rep->result_in_aux ? aux : src;
 		return RSX_OK;
 	}
-	Plan P;
-	make_plan(P, n, layout, kd, 0);
+	const Plan P = make_plan(n, layout->record_bytes, kd, 0);
 	Lease L;
-	int r = acquire(L, dev, P.total);
-	if (r)
+	if ((r = acquire(L, dev, WORKSPACE, P.total)))
 		return r;
 	L.enqueued(st);
 	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
 	const int sms = g_dev[dev].num_sms;
 	if ((r = enqueue_front(src, P, wsp, L.pinned, sms, st)))
 		return r;
-	rsx_report local;
-	if (!rep)
-		rep = &local;
 	// Key compaction (README.md:716-758) for large keys-only sorts: one early look at what K1 found.
 	// If the bits that vary over the input fit in at least two fewer 8-bit columns than the live
 	// byte columns, the keys are compacted and sorted in that many fewer passes.
@@ -804,14 +839,9 @@ static int sort_device(void *src, void *aux, size_t n, const rsx_layout *layout,
 		const Ctl first = *L.pinned;
 		Compaction cmp;
 		if (!first.early_exit && plan_compaction(first, kd, &cmp)) {
-			rep->early_exit = 0;
-			rep->ncols = first.ncols;
-			rep->live_mask = first.live_mask;
-			rep->result_in_aux = first.ncols & 1u; // the reference's rule, on ITS column count
-			rep->staged = staged;
 			if ((r = sort_compacted(src, aux, P, wsp, L, cmp, first, sms, st)))
 				return r;
-			rep->kernel_launches = (uint32_t)(g_launches.load() - l0);
+			fill_report(rep, first, l0, staged); // the reference's pass table, on ITS column count
 			rep->compacted_passes = (cmp.bits + 7) / 8;
 			*result = rep->result_in_aux ? aux : src;
 			return RSX_OK;
@@ -840,24 +870,20 @@ static int sort_device_generic(void *src, void *aux, size_t n, const rsx_layout 
 	const int idxb = n <= 0xFFFFFFFFull ? 4 : 8;
 	const rsx_layout key_layout = {kb, 0, kb, layout->kdf_kind, layout->flags};
 	const size_t kbytes = align_up(n * kb, 256);
-	StageLease SL;
-	int r = acquire_stage(SL, dev, kbytes + 2 * n * (size_t)idxb);
+	Lease SL;
+	int r = acquire(SL, dev, STAGE, kbytes + 2 * n * (size_t)idxb);
 	if (r)
 		return r;
-	SL.inflight = st;
-	SL.has_inflight = true;
+	SL.enqueued(st);
 	unsigned char *keys = static_cast<unsigned char *>(SL.ptr), *ib = keys + kbytes;
 	const int sms = g_dev[dev].num_sms;
 	CU(launch_extract_keys(src, n, rb, layout->key_offset, kb, keys, sms, st));
 	void *ranks = nullptr;
-	rsx_report local;
-	if (!rep)
-		rep = &local;
 	if ((r = rank_device(keys, ib, n, &key_layout, kdk, idxb, &ranks, rep, st, dev, staged)))
 		return r;
 	rep->kernel_launches += 1;
 	if (rep->early_exit) { // radix_sort.hpp:60-62: nothing moves
-		SL.has_inflight = false;
+		SL.drained();
 		*result = src;
 		return RSX_OK;
 	}
@@ -866,8 +892,40 @@ static int sort_device_generic(void *src, void *aux, size_t n, const rsx_layout 
 	if (!rep->result_in_aux) // even number of live columns: the reference's result is in src
 		CU(cudaMemcpyAsync(src, aux, n * (size_t)rb, cudaMemcpyDeviceToDevice, st));
 	CU(cudaStreamSynchronize(st));
-	SL.has_inflight = false;
+	SL.drained();
 	*result = rep->result_in_aux ? aux : src;
+	return RSX_OK;
+}
+
+// Host buffers: stage through device memory.  The first src_bytes of the stage lease receive src,
+// the next other_bytes are the second buffer; sort_dev(dsrc, dother, &dres) sorts there.  out_bytes
+// of the result come back to out_even, or to out_odd when the result is in the second buffer (the
+// reference's parity rule); an early exit copies nothing back unless always_copy.
+static int sort_staged(const void *src, size_t src_bytes, size_t other_bytes, void *out_even, void *out_odd, size_t out_bytes,
+                       bool always_copy, int dev, cudaStream_t st, rsx_report *rep, void **result,
+                       const std::function<int(void *, void *, void **)> &sort_dev) {
+	Lease SL;
+	int r = acquire(SL, dev, STAGE, align_up(src_bytes, 256) + other_bytes);
+	if (r)
+		return r;
+	SL.enqueued(st); // drained below on success, by ~Lease on any failure
+	unsigned char *dsrc = static_cast<unsigned char *>(SL.ptr), *dother = dsrc + align_up(src_bytes, 256);
+	cudaError_t e = cudaMemcpyAsync(dsrc, src, src_bytes, cudaMemcpyHostToDevice, st);
+	if (e != cudaSuccess)
+		return fail_cuda(e, "H2D");
+	void *dres = nullptr;
+	if ((r = sort_dev(dsrc, dother, &dres)))
+		return r;
+	void *hres = rep->result_in_aux ? out_odd : out_even;
+	if (always_copy || !rep->early_exit) {
+		e = cudaMemcpyAsync(hres, dres, out_bytes, cudaMemcpyDeviceToHost, st);
+		if (e == cudaSuccess)
+			e = cudaStreamSynchronize(st);
+		if (e != cudaSuccess)
+			return fail_cuda(e, "D2H");
+	}
+	SL.drained(); // sort_dev / the D2H copy synchronised the stream
+	*result = hres;
 	return RSX_OK;
 }
 
@@ -880,12 +938,10 @@ int rsx_sort(void *src, void *aux, size_t n, const rsx_layout *layout, void **re
 		return r;
 	if (!result || (n && (!src || !aux)))
 		return RSX_ERR_INVALID;
-	if (n >= 2) { // src and aux are __restrict__ in the reference (radix_sort.hpp:32): overlapping buffers are a bug
-		const unsigned char *a = static_cast<const unsigned char *>(src), *b = static_cast<const unsigned char *>(aux);
-		const size_t bytes = n * layout->record_bytes;
-		if (a < b + bytes && b < a + bytes)
-			return RSX_ERR_INVALID;
-	}
+	const size_t bytes = n * layout->record_bytes;
+	// src and aux are __restrict__ in the reference (radix_sort.hpp:32): overlapping buffers are a bug
+	if (n >= 2 && overlaps(src, bytes, aux, bytes))
+		return RSX_ERR_INVALID;
 	if (n < 2) { // radix_sort.hpp:100-101
 		*result = src;
 		trivial_report(rep);
@@ -894,81 +950,38 @@ int rsx_sort(void *src, void *aux, size_t n, const rsx_layout *layout, void **re
 	int dev;
 	if ((r = current_device(&dev)))
 		return r;
-	PtrKind ks, ka;
-	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(aux, &ka)))
+	PtrKind kind;
+	if ((r = check_residency(&kind, src, aux)))
 		return r;
-	if (ks != ka)
-		return RSX_ERR_MIXED_MEMORY;
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
+	rep = report_or_scratch(rep);
 	auto sort_dev = [&](void *s_, void *a_, void **res_, bool staged_) {
 		return generic ? sort_device_generic(s_, a_, n, layout, kd, res_, rep, st, dev, staged_)
 		               : sort_device(s_, a_, n, layout, kd, res_, rep, st, dev, staged_);
 	};
-	if (ks == PK_DEVICE)
+	if (kind == PK_DEVICE)
 		return sort_dev(src, aux, result, false);
-
-	// Host buffers: stage through device memory.  The reference sorts host memory in place;
-	// the bytes land in the buffer it would have returned, the other buffer is left as is
-	// (the reference leaves the penultimate pass there, which callers must treat as garbage).
-	const size_t bytes = n * layout->record_bytes;
-	StageLease SL;
-	if ((r = acquire_stage(SL, dev, 2 * align_up(bytes, 256))))
-		return r;
-	void *d = SL.ptr;
-	void *dsrc = d, *daux = static_cast<unsigned char *>(d) + align_up(bytes, 256);
-	void *dres = nullptr;
-	rsx_report local;
-	if (!rep)
-		rep = &local;
-	r = RSX_OK;
-	SL.inflight = st;
-	SL.has_inflight = true; // drained below on success, by ~StageLease on any failure
-	cudaError_t e = cudaMemcpyAsync(dsrc, src, bytes, cudaMemcpyHostToDevice, st);
-	if (e != cudaSuccess)
-		r = fail_cuda(e, "H2D");
-	if (!r)
-		r = sort_dev(dsrc, daux, &dres, true);
-	if (!r && !rep->early_exit) {
-		void *hres = rep->result_in_aux ? aux : src;
-		e = cudaMemcpyAsync(hres, dres, bytes, cudaMemcpyDeviceToHost, st);
-		if (e == cudaSuccess)
-			e = cudaStreamSynchronize(st);
-		if (e != cudaSuccess)
-			r = fail_cuda(e, "D2H");
-	}
-	if (!r) {
-		SL.has_inflight = false; // sort_device / the D2H copy synchronised the stream
-		*result = rep->result_in_aux ? aux : src;
-	}
-	return r;
+	// The reference sorts host memory in place: the bytes land in the buffer it would have returned,
+	// the other buffer is left as is (the reference leaves the penultimate pass there, which callers
+	// must treat as garbage).
+	return sort_staged(src, bytes, align_up(bytes, 256), src, aux, bytes, false, dev, st, rep, result,
+	                   [&](void *ds, void *da, void **dres) { return sort_dev(ds, da, dres, true); });
 }
 
 // ---- rank sort ---------------------------------------------------------------------------------
 static int rank_device(const void *src, void *ib, size_t n, const rsx_layout *layout, const KeyDesc &kd,
                        int idx_bytes, void **result, rsx_report *rep, cudaStream_t st, int dev, bool staged) {
 	const unsigned long long l0 = g_launches.load();
-	if (g_small_path.load(std::memory_order_relaxed) && n <= small_sort_capacity(layout->record_bytes, true)) {
-		Lease L;
-		int r = acquire(L, dev, sizeof(WsHead) + 256);
-		if (r)
-			return r;
-		L.enqueued(st);
-		prof_mark(st, true);
-		CU(launch_small_sort(src, nullptr, nullptr, ib, idx_bytes, n, layout->record_bytes, kd, L.pinned, st));
-		prof_mark(st);
-		rsx_report local;
-		if (!rep)
-			rep = &local;
-		if ((r = read_ctl(L, st, l0, rep, staged)))
+	int r;
+	if (fits_one_cta(n, layout->record_bytes, true)) {
+		if ((r = sort_one_cta(src, nullptr, nullptr, ib, idx_bytes, n, layout->record_bytes, kd, rep, st, dev, staged, l0)))
 			return r;
 		*result = static_cast<unsigned char *>(ib) + (rep->result_in_aux ? n * (size_t)idx_bytes : 0);
 		return RSX_OK;
 	}
-	Plan P;
-	make_plan(P, n, layout, kd, idx_bytes);
+	const Plan P = make_plan(n, layout->record_bytes, kd, idx_bytes);
 	Lease L;
-	int r = acquire(L, dev, P.total);
-	if (r)
+	if ((r = acquire(L, dev, WORKSPACE, P.total)))
 		return r;
 	L.enqueued(st);
 	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
@@ -997,9 +1010,6 @@ static int rank_device(const void *src, void *ib, size_t n, const rsx_layout *la
 	if (idx_bytes < 4)
 		CU(launch_narrow_index(reinterpret_cast<uint32_t *>(wsp + P.off_idx[0]),
 		                       reinterpret_cast<uint32_t *>(wsp + P.off_idx[1]), ib, idx_bytes, n, &ws->ctl, st));
-	rsx_report local;
-	if (!rep)
-		rep = &local;
 	if ((r = read_ctl(L, st, l0, rep, staged)))
 		return r;
 	*result = rep->result_in_aux ? ibb + n * (size_t)idx_bytes : ibb; // radix_sort_rank.hpp:91
@@ -1013,7 +1023,7 @@ int rsx_sort_rank(const void *src, void *index_buffer, size_t n, const rsx_layou
 	int r = check_layout_any(layout, &kd, &generic);
 	if (r)
 		return r;
-	if (!(idx_bytes == 1 || idx_bytes == 2 || idx_bytes == 4 || idx_bytes == 8))
+	if (!valid_idx_bytes(idx_bytes))
 		return RSX_ERR_INVALID;
 	if (!result || (n && (!src || !index_buffer)))
 		return RSX_ERR_INVALID;
@@ -1036,12 +1046,11 @@ int rsx_sort_rank(const void *src, void *index_buffer, size_t n, const rsx_layou
 	}
 	if ((r = current_device(&dev)))
 		return r;
-	PtrKind ks, ki;
-	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(index_buffer, &ki)))
+	PtrKind kind;
+	if ((r = check_residency(&kind, src, index_buffer)))
 		return r;
-	if (ks != ki)
-		return RSX_ERR_MIXED_MEMORY;
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
+	rep = report_or_scratch(rep);
 	// records of any size: rank the extracted keys (src itself is never written either way)
 	const rsx_layout key_layout = {layout->key_bytes, 0, layout->key_bytes, layout->kdf_kind, layout->flags};
 	auto rank_dev = [&](const void *s_, void *ib_, void **res_, bool staged_) -> int {
@@ -1057,40 +1066,13 @@ int rsx_sort_rank(const void *src, void *index_buffer, size_t n, const rsx_layou
 		cudaFreeAsync(keys, st);
 		return rr;
 	};
-	if (ks == PK_DEVICE)
+	if (kind == PK_DEVICE)
 		return rank_dev(src, index_buffer, result, false);
-
-	const size_t sbytes = n * layout->record_bytes, ibytes = n * (size_t)idx_bytes;
-	StageLease SL;
-	if ((r = acquire_stage(SL, dev, align_up(sbytes, 256) + 2 * ibytes)))
-		return r;
-	unsigned char *dsrc = static_cast<unsigned char *>(SL.ptr), *dib = dsrc + align_up(sbytes, 256);
-	void *dres = nullptr;
-	rsx_report local;
-	if (!rep)
-		rep = &local;
-	r = RSX_OK;
-	SL.inflight = st;
-	SL.has_inflight = true;
-	cudaError_t e = cudaMemcpyAsync(dsrc, src, sbytes, cudaMemcpyHostToDevice, st);
-	if (e != cudaSuccess)
-		r = fail_cuda(e, "H2D");
-	if (!r)
-		r = rank_dev(dsrc, dib, &dres, true);
-	unsigned char *hres = static_cast<unsigned char *>(index_buffer);
-	if (!r) {
-		hres += rep->result_in_aux ? ibytes : 0;
-		e = cudaMemcpyAsync(hres, dres, ibytes, cudaMemcpyDeviceToHost, st);
-		if (e == cudaSuccess)
-			e = cudaStreamSynchronize(st);
-		if (e != cudaSuccess)
-			r = fail_cuda(e, "D2H");
-	}
-	if (!r) {
-		SL.has_inflight = false;
-		*result = hres;
-	}
-	return r;
+	// the indices of an early exit are the identity, written by the device: always copied back
+	const size_t ibytes = n * (size_t)idx_bytes;
+	return sort_staged(src, n * layout->record_bytes, 2 * ibytes, index_buffer, static_cast<unsigned char *>(index_buffer) + ibytes,
+	                   ibytes, true, dev, st, rep, result,
+	                   [&](void *ds, void *dib, void **dres) { return rank_dev(ds, dib, dres, true); });
 }
 
 // ---- segmented sort ------------------------------------------------------------------------------
@@ -1127,9 +1109,10 @@ static bool is_device_memory(const void *p) {
 	return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
-// Grow-only pinned host memory of the calling thread: the device offsets are read back into it and
-// the group plan is built in it and uploaded with one copy.  The calls using it are synchronous.
-static int segment_host_buffer(size_t bytes, unsigned char **out) {
+// Grow-only pinned host memory of the calling thread: segmented sorts read the device offsets back
+// into it and build and upload their group plan in it, top-k reads back its column count.  The calls
+// using it are synchronous.
+static int thread_pinned_buffer(size_t bytes, unsigned char **out) {
 	thread_local void *buf = nullptr;
 	thread_local size_t cap = 0;
 	if (cap < bytes) {
@@ -1188,16 +1171,13 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 	int r = check_layout(layout, &kd); // records the tile kernels move directly: 1, 2, 4, 8 or 16 bytes
 	if (r)
 		return r;
-	if (ranksort && !(idx_bytes == 1 || idx_bytes == 2 || idx_bytes == 4 || idx_bytes == 8))
+	if (ranksort && !valid_idx_bytes(idx_bytes))
 		return RSX_ERR_INVALID;
 	if (!result || !offsets || (n && (!src || !(ranksort ? ib : aux))) || (nseg == 0 && n > 0))
 		return RSX_ERR_INVALID;
 	const uint32_t rb = layout->record_bytes;
-	if (!ranksort && n >= 2) {
-		const unsigned char *a = static_cast<const unsigned char *>(src), *b = static_cast<const unsigned char *>(aux);
-		if (a < b + n * rb && b < a + n * rb)
-			return RSX_ERR_INVALID;
-	}
+	if (!ranksort && n >= 2 && overlaps(src, n * rb, aux, n * rb))
+		return RSX_ERR_INVALID;
 	// host offsets: everything is checked before any device work
 	const bool dev_offsets = is_device_memory(offsets);
 	size_t max_len = 0;
@@ -1217,11 +1197,8 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 	int dev;
 	if ((r = current_device(&dev)))
 		return r;
-	PtrKind ks, kb;
-	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(ranksort ? ib : aux, &kb)))
+	if ((r = check_residency(nullptr, src, ranksort ? ib : aux)))
 		return r;
-	if (ks != PK_DEVICE || kb != PK_DEVICE)
-		return RSX_ERR_MIXED_MEMORY;
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	const unsigned long long l0 = g_launches.load();
 	const size_t off_bytes = (nseg + 1) * sizeof(uint64_t);
@@ -1230,7 +1207,7 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 	unsigned char *hbuf = nullptr;
 	const size_t rd_bytes = dev_offsets ? align_up(off_bytes, 256) : 0;
 	const size_t tab_cap = align_up(2 * nseg * sizeof(uint32_t), 256); // <= one start per segment + one end per group
-	if ((r = segment_host_buffer(rd_bytes + tab_cap + nseg * sizeof(SegGroup), &hbuf)))
+	if ((r = thread_pinned_buffer(rd_bytes + tab_cap + nseg * sizeof(SegGroup), &hbuf)))
 		return r;
 	const uint64_t *hoff = offsets;
 	if (dev_offsets) { // read back once
@@ -1257,7 +1234,7 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 		const size_t off_head = 0, off_offs = align_up(sizeof(WsHead), 256);
 		const size_t off_plan = off_offs + (dev_offsets ? 0 : align_up(off_bytes, 256));
 		Lease L;
-		if ((r = acquire(L, dev, off_plan + tab_bytes + grp_bytes)))
+		if ((r = acquire(L, dev, WORKSPACE, off_plan + tab_bytes + grp_bytes)))
 			return r;
 		L.enqueued(st);
 		unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
@@ -1283,15 +1260,14 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 	const bool early = c.early_exit != 0, odd = !early && (c.ncols & 1u);
 	// ---- long segments: the ordinary path on the sub-range, result moved where the batch's lies ----
 	if (!large.empty() && !(early && !ranksort)) {
-		StageLease SL;
+		Lease SL;
 		size_t max_large = 0;
 		for (size_t s : large)
 			max_large = hoff[s + 1] - hoff[s] > max_large ? hoff[s + 1] - hoff[s] : max_large;
 		if (ranksort) {
-			if ((r = acquire_stage(SL, dev, 2 * max_large * (size_t)idx_bytes)))
+			if ((r = acquire(SL, dev, STAGE, 2 * max_large * (size_t)idx_bytes)))
 				return r;
-			SL.inflight = st;
-			SL.has_inflight = true;
+			SL.enqueued(st);
 		}
 		for (size_t s : large) {
 			const size_t o = hoff[s], len = hoff[s + 1] - o;
@@ -1315,16 +1291,9 @@ static int sort_segments_common(const void *src, void *aux, void *ib, int idx_by
 			}
 		}
 		CU(cudaStreamSynchronize(st));
-		SL.has_inflight = false;
+		SL.drained();
 	}
-	if (rep) {
-		memset(rep, 0, sizeof(*rep));
-		rep->early_exit = early;
-		rep->ncols = early ? 0 : c.ncols;
-		rep->live_mask = early ? 0 : c.live_mask;
-		rep->result_in_aux = odd;
-		rep->kernel_launches = (uint32_t)(g_launches.load() - l0);
-	}
+	fill_report(rep, c, l0, false);
 	if (ranksort)
 		*result = static_cast<unsigned char *>(ib) + (odd ? n * (size_t)idx_bytes : 0);
 	else
@@ -1356,17 +1325,13 @@ static int topk_common(const void *src, size_t n, size_t k, const rsx_layout *la
 	int r = check_layout(layout, &kd); // records the tile kernels move directly: 1, 2, 4, 8 or 16 bytes
 	if (r)
 		return r;
-	if (ranksort && !(idx_bytes == 1 || idx_bytes == 2 || idx_bytes == 4 || idx_bytes == 8))
+	if (ranksort && !valid_idx_bytes(idx_bytes))
 		return RSX_ERR_INVALID;
 	if (k > n || (k > 0 && (!src || !out)))
 		return RSX_ERR_INVALID;
 	const uint32_t rb = layout->record_bytes;
-	if (k > 0) { // src is never written: the output must not overlap it
-		const unsigned char *a = static_cast<const unsigned char *>(src), *b = static_cast<const unsigned char *>(out);
-		const size_t ob = k * (ranksort ? (size_t)idx_bytes : rb);
-		if (a < b + ob && b < a + n * rb)
-			return RSX_ERR_INVALID;
-	}
+	if (k > 0 && overlaps(src, n * rb, out, k * (ranksort ? (size_t)idx_bytes : rb))) // src is never written
+		return RSX_ERR_INVALID;
 	if (ranksort && !idx_fits(idx_bytes, n))
 		return RSX_ERR_IDX_RANGE;
 	if (rep)
@@ -1376,11 +1341,8 @@ static int topk_common(const void *src, size_t n, size_t k, const rsx_layout *la
 	int dev;
 	if ((r = current_device(&dev)))
 		return r;
-	PtrKind ks, ko;
-	if ((r = ptr_kind(src, &ks)) || (r = ptr_kind(out, &ko)))
+	if ((r = check_residency(nullptr, src, out)))
 		return r;
-	if (ks != PK_DEVICE || ko != PK_DEVICE)
-		return RSX_ERR_MIXED_MEMORY;
 	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	const unsigned long long l0 = g_launches.load();
 	const int sms = g_dev[dev].num_sms;
@@ -1396,13 +1358,12 @@ static int topk_common(const void *src, size_t n, size_t k, const rsx_layout *la
 	const size_t off_ib = off_pos + (ranksort ? align_up(k * (size_t)sel_ib, 256) : 0);
 	const size_t total = off_ib + (ranksort ? 2 * k * (size_t)rank_ib : 0);
 	unsigned char *hbuf = nullptr;
-	if ((r = segment_host_buffer(sizeof(uint32_t), &hbuf)))
+	if ((r = thread_pinned_buffer(sizeof(uint32_t), &hbuf)))
 		return r;
-	StageLease SL;
-	if ((r = acquire_stage(SL, dev, total)))
+	Lease SL;
+	if ((r = acquire(SL, dev, STAGE, total)))
 		return r;
-	SL.inflight = st;
-	SL.has_inflight = true; // drained below on success, by ~StageLease on any failure
+	SL.enqueued(st); // drained below on success, by ~Lease on any failure
 	unsigned char *sp = static_cast<unsigned char *>(SL.ptr);
 	TopkState *s = reinterpret_cast<TopkState *>(sp);
 	auto *clt = reinterpret_cast<unsigned long long *>(sp + off_lt), *ceq = reinterpret_cast<unsigned long long *>(sp + off_eq);
@@ -1428,11 +1389,12 @@ static int topk_common(const void *src, size_t n, size_t k, const rsx_layout *la
 		CU(launch_topk_gather(res, rank_ib, sp + off_pos, sel_ib, out, idx_bytes, k, sms, st));
 	}
 	CU(cudaStreamSynchronize(st));
-	SL.has_inflight = false;
-	if (rep) {
-		rep->ncols = *reinterpret_cast<const uint32_t *>(hbuf);
-		rep->kernel_launches = (uint32_t)(g_launches.load() - l0);
-	}
+	SL.drained();
+	Ctl c{};
+	c.ncols = *reinterpret_cast<const uint32_t *>(hbuf); // the columns the threshold search histogrammed
+	fill_report(rep, c, l0, false);
+	if (rep)
+		rep->result_in_aux = 0; // the k records are always in `out`
 	return RSX_OK;
 }
 
@@ -1456,40 +1418,23 @@ int rsx_histogram(const void *src, size_t n, const rsx_layout *layout, uint64_t 
 		return r;
 	if (!src || n < 2)
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = check_residency(nullptr, src)))
 		return r;
-	PtrKind k;
-	if ((r = ptr_kind(src, &k)))
-		return r;
-	if (k != PK_DEVICE)
-		return RSX_ERR_MIXED_MEMORY;
 	const unsigned long long l0 = g_launches.load();
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	make_plan(P, n, layout, kd, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
+	if ((r = C.lease(make_plan(n, layout->record_bytes, kd, 0))))
 		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	if ((r = enqueue_front(src, P, wsp, L.pinned, g_dev[dev].num_sms, st)))
+	if ((r = enqueue_front(src, C.P, C.wsp, C.L.pinned, C.sms, C.st)))
 		return r;
-	rsx_report local;
-	if (!rep)
-		rep = &local;
-	if ((r = read_ctl(L, st, l0, rep, false)))
+	rep = report_or_scratch(rep);
+	if ((r = read_ctl(C.L, C.st, l0, rep, false)))
 		return r;
-	rep->live_mask = L.pinned->live_mask; // report the probe even when the input is presorted
-	rep->ncols = L.pinned->ncols;
-	if (hist_out) {
-		CU(cudaMemcpyAsync(L.readback(), ws->hist, sizeof(uint64_t) * kBins * kd.key_bytes, cudaMemcpyDeviceToHost, st));
-		CU(cudaStreamSynchronize(st));
-		memcpy(hist_out, L.readback(), sizeof(uint64_t) * kBins * kd.key_bytes);
-	}
-	if (descents_out)
-		CU(cudaMemcpy(descents_out, &ws->descents, sizeof(uint64_t), cudaMemcpyDeviceToHost));
+	rep->live_mask = C.L.pinned->live_mask; // report the probe even when the input is presorted
+	rep->ncols = C.L.pinned->ncols;
+	if (hist_out && (r = C.read_back(C.ws->hist, sizeof(uint64_t) * kBins * kd.key_bytes, hist_out)))
+		return r;
+	if (descents_out && (r = C.read_back(&C.ws->descents, sizeof(uint64_t), descents_out)))
+		return r;
 	return RSX_OK;
 }
 
@@ -1500,14 +1445,9 @@ int rsx_histogram_column(const void *src, size_t n, const rsx_layout *layout, in
 		return r;
 	if (!src || !hist_out || n < 1 || col < 0 || col >= (int)kd.key_bytes)
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = check_residency(nullptr, src)))
 		return r;
-	PtrKind k;
-	if ((r = ptr_kind(src, &k)))
-		return r;
-	if (k != PK_DEVICE)
-		return RSX_ERR_MIXED_MEMORY;
 	// The digit of column `col` of the derived key is the derived key of a ONE-byte key at that
 	// byte position: the top column keeps the sign / float flip (the sign bit lives in it), lower
 	// columns are plain bytes; a complemented key complements every byte.
@@ -1519,24 +1459,11 @@ int rsx_histogram_column(const void *src, size_t n, const rsx_layout *layout, in
 			return RSX_ERR_INVALID; // a lower column of a float key depends on the sign in the top byte
 		k1.kdf_kind = RSX_KDF_UNSIGNED;
 	}
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	rsx_layout l1 = *layout;
-	l1.key_bytes = 1;
-	Plan P;
-	make_plan(P, 2, &l1, k1, 0); // head only: no pass follows
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
+	if ((r = C.lease(head_plan(layout->record_bytes, k1))))
 		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	CU(zero_workspace(P, wsp, st));
-	CU(launch_histogram(src, n, layout->record_bytes, k1, ws, g_dev[dev].num_sms, st));
-	CU(cudaMemcpyAsync(L.readback(), ws->hist, sizeof(uint64_t) * kBins, cudaMemcpyDeviceToHost, st));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	memcpy(hist_out, L.readback(), sizeof(uint64_t) * kBins);
-	return RSX_OK;
+	CU(zero_workspace(C.P, C.wsp, C.st));
+	CU(launch_histogram(src, n, layout->record_bytes, k1, C.ws, C.sms, C.st));
+	return C.read_back(C.ws->hist, sizeof(uint64_t) * kBins, hist_out);
 }
 
 int rsx_scatter_pass(const void *src, void *dst, const void *payload_src, void *payload_dst,
@@ -1551,20 +1478,10 @@ int rsx_scatter_pass(const void *src, void *dst, const void *payload_src, void *
 		return RSX_ERR_INVALID;
 	if (payload_bytes && (!payload_src || !payload_dst))
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(make_plan(n, layout->record_bytes, kd, 0, payload_bytes))))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	make_plan(P, n, layout, kd, 0, payload_bytes);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	const int sms = g_dev[dev].num_sms;
-	if ((r = enqueue_front(src, P, wsp, L.pinned, sms, st))) // histogram + scan give this column's offsets
+	if ((r = enqueue_front(src, C.P, C.wsp, C.L.pinned, C.sms, C.st))) // histogram + scan give this column's offsets
 		return r;
 	PassBuffers pb{};
 	pb.rec_first = src;
@@ -1573,49 +1490,18 @@ int rsx_scatter_pass(const void *src, void *dst, const void *payload_src, void *
 	pb.pl_first = payload_src;
 	pb.pl_buf[0] = payload_dst;
 	pb.pl_buf[1] = payload_dst;
-	if ((r = run_scatter(pb, P, col, wsp, true, true, sms, st)))
+	if ((r = run_scatter(pb, C.P, col, C.wsp, true, C.sms, C.st)))
 		return r;
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	return RSX_OK;
+	return C.finish();
 }
 
-int rsx_scatter_pass_to(const void *src, size_t n, const rsx_layout *layout, int col,
-                        const uint8_t *owner, const uint64_t *dest_base, int ndest, void *stream) {
-	KeyDesc kd;
-	int r = check_layout(layout, &kd);
-	if (r)
-		return r;
-	if (!src || !owner || !dest_base || n < 1 || col < 0 || col >= (int)kd.key_bytes || ndest < 1 || ndest > kBins)
-		return RSX_ERR_INVALID;
-	for (int b = 0; b < kBins; ++b) // contiguous ranges: owner is non-decreasing and < ndest
+// ---- fused partition + exchange ------------------------------------------------------------------
+// owner: contiguous bucket ranges, non-decreasing and < ndest.
+static bool valid_owner(const uint8_t *owner, int ndest) {
+	for (int b = 0; b < kBins; ++b)
 		if (owner[b] >= ndest || (b && owner[b] < owner[b - 1]))
-			return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
-		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	make_plan(P, n, layout, kd, 0, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	const int sms = g_dev[dev].num_sms;
-	// no histogram needed: destinations get explicit base addresses; only the look-back state and
-	// the tile ticket have to be zero (the caller already histogrammed this shard to route it)
-	CU(zero_workspace(P, wsp, st));
-	CU(cudaMemcpyAsync(ws->dest_base, dest_base, sizeof(uint64_t) * ndest, cudaMemcpyHostToDevice, st));
-	CU(cudaMemcpyAsync(ws->owner, owner, kBins, cudaMemcpyHostToDevice, st));
-	PassBuffers pb{};
-	pb.rec_first = src;
-	CU(launch_scatter(pb, P.n, P.rb, 0, P.kd, col, ws, true, wsp + (size_t)col * P.status_bytes, &ws->tickets[col], P.wide, sms, st,
-	                  ws->dest_base, ws->owner, nullptr, 0, ndest));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	return RSX_OK;
+			return false;
+	return true;
 }
 
 // Key-range routing (sample-sort style splitters) for skewed multi-GPU inputs.
@@ -1628,6 +1514,65 @@ static int check_splitters(const uint64_t *splitters, int nsplit) {
 	return RSX_OK;
 }
 
+// With splitters, the "digit" of a record is its key range: range j goes to destination j.
+static void splitter_owner(int nsplit, unsigned char owner[kBins]) {
+	for (int b = 0; b < kBins; ++b)
+		owner[b] = (unsigned char)(b <= nsplit ? b : nsplit);
+}
+
+// One exchange pass over column col (key ranges when splitters != nullptr), on a workspace the caller
+// has prepared.  The HOST arrays dest_base and owner -- in append mode (dest_cursor != nullptr) also
+// dest_cursor and dest_capacity -- are uploaded into the workspace head first; append mode reads back
+// whether a run did not fit.
+static int exchange_pass(DeviceCall &C, const void *src, int col, const uint8_t *owner, const uint64_t *dest_base, int ndest,
+                         const uint64_t *splitters, int nsplit, const uint64_t *dest_cursor = nullptr,
+                         const uint64_t *dest_capacity = nullptr, uint32_t *overflow_out = nullptr) {
+	WsHead *ws = C.ws;
+	const size_t dbytes = sizeof(uint64_t) * ndest;
+	CU(cudaMemcpyAsync(ws->dest_base, dest_base, dbytes, cudaMemcpyHostToDevice, C.st));
+	if (dest_cursor) {
+		CU(cudaMemcpyAsync(ws->dest_cursor, dest_cursor, dbytes, cudaMemcpyHostToDevice, C.st));
+		CU(cudaMemcpyAsync(ws->dest_capacity, dest_capacity, dbytes, cudaMemcpyHostToDevice, C.st));
+	}
+	CU(cudaMemcpyAsync(ws->owner, owner, kBins, cudaMemcpyHostToDevice, C.st));
+	Exchange ex;
+	ex.dest_base = ws->dest_base;
+	ex.owner = ws->owner;
+	ex.splitters = reinterpret_cast<const unsigned long long *>(splitters);
+	ex.nsplit = nsplit;
+	ex.ndest = ndest;
+	if (dest_cursor) {
+		ex.dest_cursor = ws->dest_cursor;
+		ex.dest_capacity = ws->dest_capacity;
+		ex.overflow = &ws->overflow;
+	}
+	PassBuffers pb{};
+	pb.rec_first = src;
+	int r = run_scatter(pb, C.P, col, C.wsp, true, C.sms, C.st, ex);
+	if (r)
+		return r;
+	return overflow_out ? C.read_back(&ws->overflow, sizeof(uint32_t), overflow_out) : C.finish();
+}
+
+int rsx_scatter_pass_to(const void *src, size_t n, const rsx_layout *layout, int col,
+                        const uint8_t *owner, const uint64_t *dest_base, int ndest, void *stream) {
+	KeyDesc kd;
+	int r = check_layout(layout, &kd);
+	if (r)
+		return r;
+	if (!src || !owner || !dest_base || n < 1 || col < 0 || col >= (int)kd.key_bytes || ndest < 1 || ndest > kBins)
+		return RSX_ERR_INVALID;
+	if (!valid_owner(owner, ndest))
+		return RSX_ERR_INVALID;
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(make_plan(n, layout->record_bytes, kd, 0, 0))))
+		return r;
+	// no histogram needed: destinations get explicit base addresses; only the look-back state and
+	// the tile ticket have to be zero (the caller already histogrammed this shard to route it)
+	CU(zero_workspace(C.P, C.wsp, C.st));
+	return exchange_pass(C, src, col, owner, dest_base, ndest, nullptr, 0);
+}
+
 int rsx_split_counts(const void *src, size_t n, const rsx_layout *layout, const uint64_t *splitters, int nsplit,
                      uint64_t *counts_out, void *stream) {
 	KeyDesc kd;
@@ -1636,34 +1581,20 @@ int rsx_split_counts(const void *src, size_t n, const rsx_layout *layout, const 
 		return r;
 	if (!counts_out || (n && !src))
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	for (int j = 0; j <= nsplit; ++j)
 		counts_out[j] = 0;
 	if (n == 0)
 		return RSX_OK;
 	// the counters live in the (zeroed) head of the cached workspace: no allocation per call
-	rsx_layout l1 = *layout;
-	Plan P;
-	make_plan(P, 2, &l1, kd, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
+	if ((r = C.lease(head_plan(layout->record_bytes, kd))))
 		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	unsigned long long h[16] = {};
-	CU(zero_workspace(P, wsp, st));
+	CU(zero_workspace(C.P, C.wsp, C.st));
 	CU(launch_split_counts(src, n, layout->record_bytes, kd, reinterpret_cast<const unsigned long long *>(splitters),
-	                       (uint32_t)nsplit, ws->hist, g_dev[dev].num_sms, st));
-	CU(cudaMemcpyAsync(h, ws->hist, sizeof(h), cudaMemcpyDeviceToHost, st));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	for (int j = 0; j <= nsplit; ++j)
-		counts_out[j] = h[j];
-	return RSX_OK;
+	                       (uint32_t)nsplit, C.ws->hist, C.sms, C.st));
+	return C.read_back(C.ws->hist, sizeof(uint64_t) * (nsplit + 1), counts_out);
 }
 
 int rsx_split_pass_to(const void *src, size_t n, const rsx_layout *layout, const uint64_t *splitters, int nsplit,
@@ -1674,34 +1605,15 @@ int rsx_split_pass_to(const void *src, size_t n, const rsx_layout *layout, const
 		return r;
 	if (!src || !dest_base || n < 1)
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(make_plan(n, layout->record_bytes, kd, 0, 0))))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	make_plan(P, n, layout, kd, 0, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	const int sms = g_dev[dev].num_sms;
 	// no histogram needed: destinations get explicit base addresses; only the look-back state and
 	// the tile ticket have to be zero
-	CU(zero_workspace(P, wsp, st));
+	CU(zero_workspace(C.P, C.wsp, C.st));
 	unsigned char owner[kBins];
-	for (int b = 0; b < kBins; ++b)
-		owner[b] = (unsigned char)(b <= nsplit ? b : nsplit); // "digit" == destination
-	CU(cudaMemcpyAsync(ws->dest_base, dest_base, sizeof(uint64_t) * (nsplit + 1), cudaMemcpyHostToDevice, st));
-	CU(cudaMemcpyAsync(ws->owner, owner, kBins, cudaMemcpyHostToDevice, st));
-	PassBuffers pb{};
-	pb.rec_first = src;
-	CU(launch_scatter(pb, P.n, P.rb, 0, P.kd, 0, ws, true, wsp, &ws->tickets[0], P.wide, sms, st,
-	                  ws->dest_base, ws->owner, reinterpret_cast<const unsigned long long *>(splitters), nsplit, nsplit + 1));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	return RSX_OK;
+	splitter_owner(nsplit, owner);
+	return exchange_pass(C, src, 0, owner, dest_base, nsplit + 1, splitters, nsplit);
 }
 
 // Append-mode partition + exchange (keys-only records): like rsx_scatter_pass_to / rsx_split_pass_to,
@@ -1719,51 +1631,24 @@ int rsx_scatter_pass_append(const void *src, size_t n, const rsx_layout *layout,
 		return RSX_ERR_INVALID;
 	if (layout->record_bytes != kd.key_bytes)
 		return RSX_ERR_INVALID; // append order is arbitrary: only where equal records are indistinguishable
-	unsigned char own[kBins];
+	unsigned char split_owner[kBins];
 	if (col >= 0) {
-		if (!owner || col >= (int)kd.key_bytes)
+		if (!owner || col >= (int)kd.key_bytes || !valid_owner(owner, ndest))
 			return RSX_ERR_INVALID;
-		for (int b = 0; b < kBins; ++b) {
-			if (owner[b] >= ndest || (b && owner[b] < owner[b - 1]))
-				return RSX_ERR_INVALID;
-			own[b] = owner[b];
-		}
+		splitters = nullptr;
 		nsplit = 0;
 	} else {
 		if ((r = check_splitters(splitters, nsplit)) || ndest != nsplit + 1)
 			return r ? r : RSX_ERR_INVALID;
-		for (int b = 0; b < kBins; ++b)
-			own[b] = (unsigned char)(b <= nsplit ? b : nsplit); // "digit" == destination
+		splitter_owner(nsplit, split_owner);
+		owner = split_owner;
+		col = 0;
 	}
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(make_plan(n, layout->record_bytes, kd, 0, 0))))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	make_plan(P, n, layout, kd, 0, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	const int sms = g_dev[dev].num_sms;
-	CU(cudaMemsetAsync(wsp + P.off_head, 0, kWsZeroBytes, st)); // ticket + overflow flag; no look-back state in this mode
-	CU(cudaMemcpyAsync(ws->dest_base, dest_base, sizeof(uint64_t) * ndest, cudaMemcpyHostToDevice, st));
-	CU(cudaMemcpyAsync(ws->dest_cursor, dest_cursor, sizeof(uint64_t) * ndest, cudaMemcpyHostToDevice, st));
-	CU(cudaMemcpyAsync(ws->dest_capacity, dest_capacity, sizeof(uint64_t) * ndest, cudaMemcpyHostToDevice, st));
-	CU(cudaMemcpyAsync(ws->owner, own, kBins, cudaMemcpyHostToDevice, st));
-	PassBuffers pb{};
-	pb.rec_first = src;
-	const int c = col >= 0 ? col : 0;
-	CU(launch_scatter(pb, P.n, P.rb, 0, P.kd, c, ws, true, wsp + (size_t)c * P.status_bytes, &ws->tickets[c], P.wide, sms, st,
-	                  ws->dest_base, ws->owner, col >= 0 ? nullptr : reinterpret_cast<const unsigned long long *>(splitters),
-	                  nsplit, ndest, ws->dest_cursor, ws->dest_capacity, &ws->overflow));
-	CU(cudaMemcpyAsync(L.readback(), &ws->overflow, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	*overflow_out = *reinterpret_cast<unsigned int *>(L.readback());
-	return RSX_OK;
+	CU(cudaMemsetAsync(C.ws, 0, kWsZeroBytes, C.st)); // ticket + overflow flag; no look-back state in this mode
+	return exchange_pass(C, src, col, owner, dest_base, ndest, splitters, nsplit, dest_cursor, dest_capacity, overflow_out);
 }
 
 // `count` evenly spaced records' DERIVED keys (record i * (n / count)), HOST output: the sample the
@@ -1775,24 +1660,11 @@ int rsx_sample_keys(const void *src, size_t n, const rsx_layout *layout, size_t 
 		return r;
 	if (!src || !derived_out || count < 1 || count > n || count > kMaxCols * kBins)
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(head_plan(layout->record_bytes, kd))))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	rsx_layout l1 = *layout;
-	make_plan(P, 2, &l1, kd, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	WsHead *ws = reinterpret_cast<WsHead *>(static_cast<unsigned char *>(L.ptr) + P.off_head);
-	CU(launch_sample_keys(src, count, n / count, layout->record_bytes, kd, ws->offs, st)); // offs: 16 KB of scratch in the head
-	CU(cudaMemcpyAsync(L.readback(), ws->offs, sizeof(uint64_t) * count, cudaMemcpyDeviceToHost, st));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	memcpy(derived_out, L.readback(), sizeof(uint64_t) * count);
-	return RSX_OK;
+	CU(launch_sample_keys(src, count, n / count, layout->record_bytes, kd, C.ws->offs, C.st)); // offs: 16 KB of scratch in the head
+	return C.read_back(C.ws->offs, sizeof(uint64_t) * count, derived_out);
 }
 
 // The 256-bin histogram of one column over a SAMPLE of the records (every stride-th one): what
@@ -1805,26 +1677,12 @@ int rsx_histogram_column_sampled(const void *src, size_t n, const rsx_layout *la
 		return r;
 	if (!src || !hist_out || n < 1 || stride < 1 || col < 0 || col >= (int)kd.key_bytes)
 		return RSX_ERR_INVALID;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)) || (r = C.lease(head_plan(layout->record_bytes, kd))))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
-	Plan P;
-	rsx_layout l1 = *layout;
-	make_plan(P, 2, &l1, kd, 0);
-	Lease L;
-	if ((r = acquire(L, dev, P.total)))
-		return r;
-	L.enqueued(st);
-	unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-	WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-	CU(zero_workspace(P, wsp, st));
-	CU(launch_sample_column_hist(src, n, layout->record_bytes, kd, col, stride, ws->hist, g_dev[dev].num_sms, st));
-	CU(cudaMemcpyAsync(L.readback(), ws->hist, sizeof(uint64_t) * kBins, cudaMemcpyDeviceToHost, st));
-	CU(cudaStreamSynchronize(st));
-	L.drained();
-	memcpy(hist_out, L.readback(), sizeof(uint64_t) * kBins);
-	return RSX_OK;
+	CU(zero_workspace(C.P, C.wsp, C.st));
+	CU(launch_sample_column_hist(src, n, layout->record_bytes, kd, col, stride, C.ws->hist, C.sms, C.st));
+	return C.read_back(C.ws->hist, sizeof(uint64_t) * kBins, hist_out);
 }
 
 // The key-compaction plan for given OR / NAND masks (pure host arithmetic; tests/test_abi.py checks
@@ -1871,25 +1729,17 @@ int rsx_verify(const void *data, size_t n, const rsx_layout *layout, uint64_t *d
 	int r = check_layout(layout, &kd);
 	if (r)
 		return r;
-	int dev;
-	if ((r = current_device(&dev)))
+	DeviceCall C;
+	if ((r = C.open(stream)))
 		return r;
-	cudaStream_t st = static_cast<cudaStream_t>(stream);
 	unsigned long long h3[3] = {0, 0, 0};
 	if (n) { // the three accumulators live in the (zeroed) head of the cached workspace
-		Plan P;
-		make_plan(P, 2, layout, kd, 0);
-		Lease L;
-		if ((r = acquire(L, dev, P.total)))
+		if ((r = C.lease(head_plan(layout->record_bytes, kd))))
 			return r;
-		L.enqueued(st);
-		unsigned char *wsp = static_cast<unsigned char *>(L.ptr);
-		WsHead *ws = reinterpret_cast<WsHead *>(wsp + P.off_head);
-		CU(zero_workspace(P, wsp, st));
-		CU(launch_verify(data, n, layout->record_bytes, kd, ws->hist, g_dev[dev].num_sms, st));
-		CU(cudaMemcpyAsync(h3, ws->hist, sizeof(h3), cudaMemcpyDeviceToHost, st));
-		CU(cudaStreamSynchronize(st));
-		L.drained();
+		CU(zero_workspace(C.P, C.wsp, C.st));
+		CU(launch_verify(data, n, layout->record_bytes, kd, C.ws->hist, C.sms, C.st));
+		if ((r = C.read_back(C.ws->hist, sizeof(h3), h3)))
+			return r;
 	}
 	if (descents_out) *descents_out = h3[0];
 	if (sum_out) *sum_out = h3[1];

@@ -107,15 +107,23 @@ cudaError_t launch_expand_keys(const void *in, void *out, size_t n, const KeyDes
 cudaError_t launch_setup(const void *src, size_t n, uint32_t record_bytes, const KeyDesc &kd,
                          WsHead *ws, Ctl *host_ctl, cudaStream_t st);
 
+// Fused partition + exchange (rsx_scatter_pass_to / rsx_split_pass_to / rsx_scatter_pass_append):
+// device copies of the routing tables.  dest_base == nullptr: an ordinary pass.
+struct Exchange {
+	const unsigned long long *dest_base = nullptr; // one byte address per destination
+	const unsigned char *owner = nullptr;          // the destination of every bucket
+	const unsigned long long *splitters = nullptr; // HOST array: key-range routing instead of digits
+	int nsplit = 0, ndest = 0;
+	const unsigned long long *dest_cursor = nullptr, *dest_capacity = nullptr; // append mode
+	unsigned int *overflow = nullptr;                                           // append mode
+};
+
 // status: look-back words for this column, tiles * 256 entries of 4 (n < 2^30) or 8 bytes, zeroed.
 // ctl == nullptr: forced pass (ordinal 0, never skipped) for rsx_scatter_pass.
 cudaError_t launch_scatter(const PassBuffers &pb, size_t n, uint32_t record_bytes, int payload_bytes,
                            const KeyDesc &kd, int col, const WsHead *ws_offsets /*offs + ctl*/,
                            bool forced, void *status, unsigned int *ticket, bool wide_offsets,
-                           int num_sms, cudaStream_t st, const unsigned long long *dest_base = nullptr,
-                           const unsigned char *owner = nullptr, const unsigned long long *splitters = nullptr,
-                           int nsplit = 0, int ndest = 0, const unsigned long long *dest_cursor = nullptr,
-                           const unsigned long long *dest_capacity = nullptr, unsigned int *overflow = nullptr);
+                           int num_sms, cudaStream_t st, const Exchange &ex);
 
 PassGeometry scatter_geometry(uint32_t record_bytes, int payload_bytes);
 

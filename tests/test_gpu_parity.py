@@ -3,6 +3,7 @@ committed golden digests of the unmodified reference.  Bit-exact: this is intege
 
 Run on the B200 box: python -m pytest tests -m gpu
 """
+import contextlib
 import json
 import os
 
@@ -593,6 +594,9 @@ def test_records_of_any_size(rsx, torch, oracle, tname, n, dist, mask):
         res = rsx.radix_sort(src, aux, None, kf_for(rsx, tname))
         want, _, _ = oracle.radix_sort(data, t.layout())
         assert res.numpy().tobytes() == want.tobytes()
+        ib = torch.full((2 * n,), -1, dtype=torch.int32)
+        hranks = rsx.radix_sort_rank(torch.from_numpy(raw.copy()), ib, None, kf_for(rsx, tname))
+        assert np.array_equal(hranks.numpy().view(np.uint32), wr)
 
 
 @pytest.mark.parametrize("tname,mask,orv,ncols,cpasses", [
@@ -677,8 +681,20 @@ def test_single_cta_capacity_boundary(rsx, torch, oracle, tname):
 
 # ---- boundary behaviour: threads, managed memory, overlapping buffers ------------------------------------
 
-def test_concurrent_host_threads(rsx, torch, oracle):
-    """SURVEY §8b: safe to call from several host threads (per-call workspace, no global mutable state)."""
+def host_sort(rsx, torch, tname, data):
+    """Value sort of CPU tensors: staged through device memory."""
+    raw = np.ascontiguousarray(data).view(np.uint8).reshape(-1)
+    src = torch.from_numpy(raw.copy())
+    aux = torch.zeros_like(src)
+    rep = rsx.RsxReport()
+    res = rsx.radix_sort(src, aux, None, kf_for(rsx, tname), report=rep)
+    assert rep.staged == 1
+    return res.numpy()
+
+
+def sort_from_threads(oracle, sort, context):
+    """Four host threads sorting at once, five times each inside context(); sort(tname, data) -> sorted
+    records."""
     import threading
     results, errors = {}, []
 
@@ -686,9 +702,9 @@ def test_concurrent_host_threads(rsx, torch, oracle):
         try:
             t = TYPES["u32" if k % 2 == 0 else "u64"]
             data = make_input(t.name, 400000 + 1000 * k, 100 + k)
-            with torch.cuda.stream(torch.cuda.Stream()):
+            with context():
                 for _ in range(5):
-                    out, rep, _ = gpu_sort(rsx, torch, t.name, data)
+                    out = sort(t.name, data)
             want, _, _ = oracle.radix_sort(data, t.layout())
             results[k] = out.tobytes() == want.tobytes()
         except Exception as e:  # noqa: BLE001
@@ -701,6 +717,31 @@ def test_concurrent_host_threads(rsx, torch, oracle):
         th.join()
     assert not errors, errors
     assert all(results.get(k) for k in range(4)), results
+
+
+def test_concurrent_host_threads(rsx, torch, oracle):
+    """SURVEY §8b: safe to call from several host threads (per-call workspace, no global mutable state)."""
+    sort_from_threads(oracle, lambda tname, data: gpu_sort(rsx, torch, tname, data)[0],
+                      lambda: torch.cuda.stream(torch.cuda.Stream()))
+
+
+def test_concurrent_host_threads_on_host_buffers(rsx, torch, oracle):
+    """Four threads staging CPU tensors at once: one holds the cached staging buffer, the others
+    stage through buffers of their own."""
+    sort_from_threads(oracle, lambda tname, data: host_sort(rsx, torch, tname, data), contextlib.nullcontext)
+
+
+def test_release_while_idle(rsx, torch, oracle):
+    """rsx_release frees the idle cached workspace and staging buffer; the next device sort and
+    host-staged sort allocate them again."""
+    t = TYPES["u64"]
+    data = make_input("u64", 300007, 29)
+    want, _, _ = oracle.radix_sort(data, t.layout())
+    assert host_sort(rsx, torch, "u64", data).tobytes() == want.tobytes()  # the staging buffer is cached now
+    rsx.reserve(64 << 20)
+    rsx.lib().rsx_release()
+    assert gpu_sort(rsx, torch, "u64", data)[0].tobytes() == want.tobytes()
+    assert host_sort(rsx, torch, "u64", data).tobytes() == want.tobytes()
 
 
 def test_managed_memory_is_sorted_in_place(rsx, torch, oracle):
